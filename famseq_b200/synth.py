@@ -216,6 +216,58 @@ def random_pedigree(seed: int, n_target: int, loops: bool = False, shuffle: bool
     return ped
 
 
+def sibship(n_children: int) -> PedFile:
+    """One couple (father 1, mother 2) and `n_children` full sibs of mixed sexes."""
+    return _mk([(1, 0, 0, 1), (2, 0, 0, 2)] + [(3 + k, 2, 1, 1 + (k % 3 == 1)) for k in range(n_children)])
+
+
+def many_spouses(n_spouses: int = 5) -> PedFile:
+    """A man (1) with `n_spouses` wives, two or three children with each; one son has a family of his own."""
+    rows = [(1, 0, 0, 1)]
+    nxt = 2
+    for w in range(n_spouses):
+        wife = nxt
+        rows.append((wife, 0, 0, 2))
+        nxt += 1
+        for k in range(2 + w % 2):
+            rows.append((nxt, wife, 1, 1 + (nxt % 2)))
+            nxt += 1
+    son = next(r[0] for r in rows if r[2] == 1 and r[3] == 1)
+    rows += [(nxt, 0, 0, 2), (nxt + 1, nxt, son, 1), (nxt + 2, nxt, son, 2)]
+    return _mk(rows)
+
+
+def three_generations(sibs: int = 8) -> PedFile:
+    """A sibship of `sibs` in each of three generations: one son of each sibship marries a founder and has the next."""
+    rows, father, mother, nxt = [(1, 0, 0, 1), (2, 0, 0, 2)], 1, 2, 3
+    for gen in range(3):
+        kids = [(nxt + k, mother, father, 1 + (k % 2 == 0)) for k in range(sibs)]
+        rows += kids
+        nxt += sibs
+        if gen < 2:
+            father = next(r[0] for r in kids if r[3] == 1)
+            mother = nxt
+            rows.append((mother, 0, 0, 2))
+            nxt += 1
+    return _mk(rows)
+
+
+def forest(families, shuffle_seed=None):
+    """Several unrelated families in one ped file: ids of family f are offset past those of the families before it.
+    Returns (ped, rows): rows[f] are the ped rows of family f in the file's order (with `shuffle_seed`, the rows of all
+    families are interleaved at random)."""
+    out, fam, base = [], [], 0
+    for f, p in enumerate(families):
+        off = lambda i: i + base if i else 0
+        out += [(off(i), off(m), off(fa), g) for i, m, fa, g in zip(p.ids, p.mids, p.fids, p.genders)]
+        fam += [f] * p.n
+        base += max(p.ids)
+    order = np.arange(len(out)) if shuffle_seed is None else np.random.default_rng(shuffle_seed).permutation(len(out))
+    ped = _mk([out[i] for i in order])
+    fam = np.asarray(fam)[order]
+    return ped, [np.nonzero(fam == f)[0] for f in range(len(families))]
+
+
 PEDIGREES = {"trio": trio, "ped14": ped14, "ped40": ped40, "half_sibs": half_sibs, "three_wives": three_wives, "ped100": ped100,
              "cousins_loop": cousins_loop}
 
