@@ -273,6 +273,8 @@ ColumnMap map_columns(const std::vector<sv> &names, size_t first, const PedRows 
 // The engine of a run: ONE fs_engine, over one GPU or (fs_create_multi) over several -- every batch is then cut into
 // contiguous slices, one per device, inside the engine (variants are independent; the Gibbs sampler's streams are
 // keyed by the global variant index, so the output does not depend on the number of devices).
+constexpr size_t kMaxPedigreeMembers = 128; // fs_create's limit
+
 struct Engine {
     fs_engine *h = nullptr;
     ~Engine() { fs_destroy(h); }
@@ -288,7 +290,10 @@ struct Engine {
             fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
         fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), (int32_t)cm.engine_cols.size(),
                        cm.engine_cols.data()};
-        if (fs_create_multi(&fp, &prm, devices.data(), (int)devices.size(), &h) != FS_OK) {
+        // ped files past the 128 members of one pedigree: a cohort of nuclear families and lone individuals (ES only)
+        const int rc = id.size() > kMaxPedigreeMembers ? fs_create_families(&fp, &prm, devices.data(), (int)devices.size(), &h)
+                                                       : fs_create_multi(&fp, &prm, devices.data(), (int)devices.size(), &h);
+        if (rc != FS_OK) {
             std::cout << fs_last_error() << std::endl;
             g_engine_failed = true;
             return false;
@@ -743,7 +748,8 @@ bool check_family(const PedRows &ped) {
         fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
     fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), 0, nullptr};
     fs_engine *h = nullptr;
-    const int rc = fs_create(&fp, nullptr, -1, &h);
+    const int host_only = -1;
+    const int rc = id.size() > kMaxPedigreeMembers ? fs_create_families(&fp, nullptr, &host_only, 1, &h) : fs_create(&fp, nullptr, -1, &h);
     fs_destroy(h);
     if (rc == FS_OK) return true;
     if (rc == FS_E_GENDER)

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../../include/famseq_b200.h"
+#include "../host/families.hpp"
 #include "../host/format_g.hpp"
 #include "../host/pedigree.hpp"
 #include "es_jit.hpp"
@@ -157,6 +158,11 @@ struct fs_engine {
     double last_kernel_ms = 0;
 
     std::vector<fs_engine *> parts; // fs_create_multi: one single-device engine per GPU (this one then has device -1)
+
+    // fs_create_families: a cohort of nuclear families and lone individuals, ES only (es_families_kernel.cu)
+    bool families = false;
+    FamilyTable fam_table;
+    FamiliesParams fam; // its device arrays are owned by this engine
 };
 
 extern "C" {
@@ -235,12 +241,16 @@ void fs_destroy(fs_engine *e) {
         cudaFree(e->d_fixups);
         cudaFree(e->d_fixes);
         cudaFree(e->d_n_fixes);
+        cudaFree(const_cast<int32_t *>(e->fam.fam_col));
+        cudaFree(const_cast<uint8_t *>(e->fam.fam_male));
+        cudaFree(const_cast<uint8_t *>(e->fam.col_male));
     }
     delete e;
 }
 
-int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_engine **out) {
-    if (!ped || !out) return fail(FS_E_ARG, "fs_create: null argument");
+// fs_create (families == false) and fs_create_families on one device (-1: host side only).
+static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, fs_engine **out) {
+    if (!ped || !out) return fail(FS_E_ARG, families ? "fs_create_families: null argument" : "fs_create: null argument");
     *out = nullptr;
     fs_params prm;
     if (params)
@@ -256,7 +266,7 @@ int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_en
         delete e;
         return fail(rc, err);
     }
-    if (e->ped.n > FS_MAX_MEMBERS) {
+    if (!families && e->ped.n > FS_MAX_MEMBERS) {
         delete e;
         return fail(FS_E_TOO_LARGE, "pedigree has more than " + std::to_string(FS_MAX_MEMBERS) + " members");
     }
@@ -274,7 +284,8 @@ int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_en
     C.lrc = prm.lrc;
     C.n = e->ped.n;
     C.s = e->ped.s();
-    for (int c = 0; c < C.s; c++) C.col_male[c] = (uint8_t)e->ped.male[e->ped.cols[c]];
+    if (!families)
+        for (int c = 0; c < C.s; c++) C.col_male[c] = (uint8_t)e->ped.male[e->ped.cols[c]];
     // calPostProbSingle fails the variant when ANY member's row sum is <= 0 (family.cpp:1433-1439);
     // for unsequenced members (lk = 1,1,1) that depends only on the prior vector in use.
     for (int f = 0; f < 4; f++) {
@@ -292,55 +303,76 @@ int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_en
         C.unseq_fail[f] = bad;
     }
 
-    // ---- pedigree compilers ----------------------------------------------------------------------
-    e->es.C = C;
-    e->es_rc = compile_es_program(e->ped, e->es.prog, e->es_err);
-    { // nuclear family: exactly two founders who are the parents of every other member, nobody else has children
-        const Pedigree &p = e->ped;
-        int father = -1, mother = -1;
-        bool ok = p.n >= 3 && p.n <= 2 + ES_NUCLEAR_MAX_CHILDREN && p.n_founders() == 2;
-        for (int i = 0; ok && i < p.n; i++)
-            if (!p.founder(i)) {
-                if (father < 0) {
-                    father = p.father[i];
-                    mother = p.mother[i];
-                }
-                ok = p.father[i] == father && p.mother[i] == mother && p.children[i].empty();
-            }
-        ok = ok && father >= 0 && p.founder(father) && p.founder(mother);
-        if (ok) {
-            NuclearParams &np = e->nuclear;
-            std::memset(&np, 0, sizeof np);
-            np.C = C;
-            np.col_father = p.col_of[father];
-            np.col_mother = p.col_of[mother];
-            for (int i = 0; i < p.n; i++)
-                if (!p.founder(i)) {
-                    np.col_child[np.n_children] = p.col_of[i];
-                    np.male_child[np.n_children] = p.male[i];
-                    np.n_children++;
-                }
-            e->is_nuclear = true;
-            np.allow_ident = 1;
-            if (const char *env = std::getenv("FAMSEQ_ES_IDENT")) np.allow_ident = env[0] != '0';
-            np.stream_tiles = 0;
-            if (const char *env = std::getenv("FAMSEQ_ES_STREAM")) np.stream_tiles = std::max(-1, std::min(1 << 20, std::atoi(env)));
-        }
-        const char *env = std::getenv("FAMSEQ_ES_GENERIC");
-        e->force_generic_es = env && env[0] == '1';
-    }
-    e->bn.C = C;
-    e->bn_rc = build_bn_plan(e->ped, e->bn.plan, e->bn_err);
-    e->mcmc.C = C;
-    e->mcmc_rc = build_mcmc_plan(e->ped, e->mcmc.plan, e->mcmc_err);
-    if (const char *env = std::getenv("FAMSEQ_MCMC_JIT")) e->jit.mode = env[0] == '0' ? 0 : (env[0] == '1' ? 1 : 2);
-    if (const char *env = std::getenv("FAMSEQ_JIT_MIN_WORK")) e->jit.min_work = std::atof(env);
-    if (const char *env = std::getenv("FAMSEQ_ES_JIT")) e->es_jit.mode = env[0] == '0' ? 0 : (env[0] == '1' ? 1 : 2);
-    if (const char *env = std::getenv("FAMSEQ_MCMC_BLOCKS")) e->mcmc_tune.blocks_cap = std::max(1, std::atoi(env));
-    if (const char *env = std::getenv("FAMSEQ_MCMC_WGLOBAL")) e->mcmc_tune.wglobal = env[0] == '1';
     // PL decode table: exactly the expression of the reference's VCF driver (file.cpp:588-590), evaluated by the host's libm
     e->pl_table.resize(FS_PL_TABLE_SIZE);
     for (int k = 0; k < FS_PL_TABLE_SIZE; k++) e->pl_table[k] = std::pow(10.0, -std::fabs((double)k) / 10.0);
+    if (families) {
+        rc = build_families(e->ped, ped->id, e->fam_table, err);
+        if (rc != FS_OK) {
+            delete e;
+            return fail(rc, err);
+        }
+        e->families = true;
+        const FamilyTable &t = e->fam_table;
+        e->fam.C = C;
+        e->fam.n_families = t.n_families();
+        e->fam.nc_max = t.nc_max;
+        e->fam.group = es_families_group(C.s);
+        std::memcpy(e->fam.class_end, t.class_end, sizeof t.class_end);
+        e->bn_rc = e->mcmc_rc = FS_E_TOO_LARGE;
+        e->bn_err = e->mcmc_err = "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(t.n_families()) +
+                                  " families: only Elston-Stewart (-method 2) runs on ped files over " +
+                                  std::to_string(FS_MAX_MEMBERS) + " members";
+    }
+
+    // ---- pedigree compilers ----------------------------------------------------------------------
+    if (!families) {
+        e->es.C = C;
+        e->es_rc = compile_es_program(e->ped, e->es.prog, e->es_err);
+        { // nuclear family: exactly two founders who are the parents of every other member, nobody else has children
+            const Pedigree &p = e->ped;
+            int father = -1, mother = -1;
+            bool ok = p.n >= 3 && p.n <= 2 + ES_NUCLEAR_MAX_CHILDREN && p.n_founders() == 2;
+            for (int i = 0; ok && i < p.n; i++)
+                if (!p.founder(i)) {
+                    if (father < 0) {
+                        father = p.father[i];
+                        mother = p.mother[i];
+                    }
+                    ok = p.father[i] == father && p.mother[i] == mother && p.children[i].empty();
+                }
+            ok = ok && father >= 0 && p.founder(father) && p.founder(mother);
+            if (ok) {
+                NuclearParams &np = e->nuclear;
+                std::memset(&np, 0, sizeof np);
+                np.C = C;
+                np.col_father = p.col_of[father];
+                np.col_mother = p.col_of[mother];
+                for (int i = 0; i < p.n; i++)
+                    if (!p.founder(i)) {
+                        np.col_child[np.n_children] = p.col_of[i];
+                        np.male_child[np.n_children] = p.male[i];
+                        np.n_children++;
+                    }
+                e->is_nuclear = true;
+                np.allow_ident = 1;
+                if (const char *env = std::getenv("FAMSEQ_ES_IDENT")) np.allow_ident = env[0] != '0';
+                np.stream_tiles = 0;
+                if (const char *env = std::getenv("FAMSEQ_ES_STREAM")) np.stream_tiles = std::max(-1, std::min(1 << 20, std::atoi(env)));
+            }
+            const char *env = std::getenv("FAMSEQ_ES_GENERIC");
+            e->force_generic_es = env && env[0] == '1';
+        }
+        e->bn.C = C;
+        e->bn_rc = build_bn_plan(e->ped, e->bn.plan, e->bn_err);
+        e->mcmc.C = C;
+        e->mcmc_rc = build_mcmc_plan(e->ped, e->mcmc.plan, e->mcmc_err);
+        if (const char *env = std::getenv("FAMSEQ_MCMC_JIT")) e->jit.mode = env[0] == '0' ? 0 : (env[0] == '1' ? 1 : 2);
+        if (const char *env = std::getenv("FAMSEQ_JIT_MIN_WORK")) e->jit.min_work = std::atof(env);
+        if (const char *env = std::getenv("FAMSEQ_ES_JIT")) e->es_jit.mode = env[0] == '0' ? 0 : (env[0] == '1' ? 1 : 2);
+        if (const char *env = std::getenv("FAMSEQ_MCMC_BLOCKS")) e->mcmc_tune.blocks_cap = std::max(1, std::atoi(env));
+        if (const char *env = std::getenv("FAMSEQ_MCMC_WGLOBAL")) e->mcmc_tune.wglobal = env[0] == '1';
+    }
 
     if (device >= 0) {
         cudaError_t crc = cudaSetDevice(device);
@@ -358,7 +390,7 @@ int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_en
         }
         e->smem_limit = prop.sharedMemPerBlockOptin;
         e->sm_count = prop.multiProcessorCount;
-        if (e->es_rc == FS_OK) {
+        if (e->es_rc == FS_OK && !families) {
             e->es_tb = es_pick_block(e->es, e->smem_limit);
             if (e->es_tb == 0) {
                 e->es_rc = FS_E_TOO_LARGE;
@@ -376,25 +408,47 @@ int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_en
                 e->mcmc_err = "pedigree too large for the MCMC kernel: chain state exceeds shared memory";
             }
         }
+        if (families) { // the family table, structure-of-arrays
+            const FamilyTable &t = e->fam_table;
+            std::vector<uint8_t> col_male((size_t)C.s);
+            for (int c = 0; c < C.s; c++) col_male[c] = (uint8_t)e->ped.male[e->ped.cols[c]];
+            int32_t *d_col = nullptr;
+            uint8_t *d_male = nullptr, *d_col_male = nullptr;
+            crc = cudaMalloc(&d_col, std::max<size_t>(t.col.size(), 1) * sizeof(int32_t));
+            if (crc == cudaSuccess) e->fam.fam_col = d_col, crc = cudaMalloc(&d_male, std::max<size_t>(t.male.size(), 1));
+            if (crc == cudaSuccess) e->fam.fam_male = d_male, crc = cudaMalloc(&d_col_male, std::max<size_t>(col_male.size(), 1));
+            if (crc == cudaSuccess) e->fam.col_male = d_col_male, crc = cudaMemcpy(d_col, t.col.data(), t.col.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+            if (crc == cudaSuccess) crc = cudaMemcpy(d_male, t.male.data(), t.male.size(), cudaMemcpyHostToDevice);
+            if (crc == cudaSuccess) crc = cudaMemcpy(d_col_male, col_male.data(), col_male.size(), cudaMemcpyHostToDevice);
+            if (crc != cudaSuccess) {
+                fs_destroy(e); // releases what was allocated
+                return cuda_fail(crc, "fs_create_families: family table upload");
+            }
+        }
     }
     *out = e;
     return FS_OK;
 }
 
-int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    if (!ped || !out || !devices || ndev < 1) return fail(FS_E_ARG, "fs_create_multi: null argument or no device");
+int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_engine **out) {
+    return create_engine(ped, params, device, false, out);
+}
+
+static int create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, bool families, fs_engine **out) {
+    const char *who = families ? "fs_create_families" : "fs_create_multi";
+    if (!ped || !out || !devices || ndev < 1) return fail(FS_E_ARG, std::string(who) + ": null argument or no device");
     *out = nullptr;
     // a device may be listed more than once: every entry gets its own pipeline (streams, buffers) on that GPU
     for (int g = 0; g < ndev; g++)
-        if (devices[g] < 0) return fail(FS_E_ARG, "fs_create_multi: negative device");
-    if (ndev == 1) return fs_create(ped, params, devices[0], out);
+        if (devices[g] < 0 && !(families && ndev == 1)) return fail(FS_E_ARG, std::string(who) + ": negative device");
+    if (ndev == 1) return create_engine(ped, params, devices[0], families, out);
     // the front engine holds the host side (pedigree, tables, info); the parts own the GPUs
     fs_engine *front = nullptr;
-    int rc = fs_create(ped, params, -1, &front);
+    int rc = create_engine(ped, params, -1, families, &front);
     if (rc != FS_OK) return rc;
     for (int g = 0; g < ndev; g++) {
         fs_engine *part = nullptr;
-        rc = fs_create(ped, params, devices[g], &part);
+        rc = create_engine(ped, params, devices[g], families, &part);
         if (rc != FS_OK) {
             const std::string keep = g_last_error;
             fs_destroy(front);
@@ -403,6 +457,24 @@ int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *
         front->parts.push_back(part);
     }
     *out = front;
+    return FS_OK;
+}
+
+int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
+    return create_multi(ped, params, devices, ndev, false, out);
+}
+
+int fs_create_families(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
+    return create_multi(ped, params, devices, ndev, true, out);
+}
+
+int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children) {
+    if (!e) return fail(FS_E_ARG, "fs_get_families: null engine");
+    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families");
+    const FamilyTable &t = e->fam_table;
+    if (family) std::memcpy(family, t.family_of.data(), t.family_of.size() * sizeof(int32_t));
+    if (n_families) *n_families = t.n_families();
+    if (n_children) std::memcpy(n_children, t.n_children.data(), t.n_children.size() * sizeof(int32_t));
     return FS_OK;
 }
 
@@ -453,8 +525,14 @@ int fs_get_tables(const fs_engine *e, double *pcp2, double *pcp2_xf, double *pcp
     return FS_OK;
 }
 
+static int no_es_program(const fs_engine *e) {
+    return fail(FS_E_TOO_LARGE, "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(e->fam_table.n_families()) +
+                                    " families: peeled by the cohort kernel, which has no message program");
+}
+
 int fs_get_es_program(const fs_engine *e, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots) {
     if (!e) return fail(FS_E_ARG, "fs_get_es_program: null engine");
+    if (e->families) return no_es_program(e);
     if (e->es_rc != FS_OK && e->es_rc != FS_E_TOO_LARGE) return fail(e->es_rc, e->es_err);
     const EsProgram &p = e->es.prog;
     if (n_words) *n_words = p.n_words;
@@ -489,6 +567,7 @@ int fs_get_gibbs_kernel(const fs_engine *e, int compile, char *text, size_t capa
 
 int fs_get_es_kernel(const fs_engine *e, int compile, char *text, size_t capacity, size_t *text_len, size_t *cubin_bytes) {
     if (!e) return fail(FS_E_ARG, "fs_get_es_kernel: null engine");
+    if (e->families) return no_es_program(e);
     if (e->es_rc != FS_OK) return fail(e->es_rc, e->es_err);
     if (!es_jit_fits(e->es, 227 * 1024))
         return fail(FS_E_TOO_LARGE, "pedigree too large for the generated ES kernel (the interpreter is used)");
@@ -662,6 +741,11 @@ static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t
         const int rc = ensure_pl_table(e, stream);
         if (rc != FS_OK) return rc;
         B.lut = e->d_pl_table;
+    }
+    if (method == FS_METHOD_ES && e->families) {
+        FS_CUDA(launch_es_families(e->fam, B, stream));
+        e->launches++;
+        return FS_OK;
     }
     const bool tma_ok = ((reinterpret_cast<uintptr_t>(B.gt) | reinterpret_cast<uintptr_t>(B.status) | reinterpret_cast<uintptr_t>(B.pl)) & 15u) == 0;
     if (method == FS_METHOD_ES && e->is_nuclear && tma_ok && !e->force_generic_es) {
@@ -845,11 +929,14 @@ static int run_host_one(fs_engine *e, int method, int64_t V, const BatchIo &io, 
     const size_t S = (size_t)e->ped.s();
     // Chunks of ~48 MB of FP64 likelihoods (a multiple of 1024 variants keeps every tile 16-byte aligned)
     // are cycled through kPipelineDepth streams so that the H2D copy of chunk k+1, the kernel of
-    // chunk k and the D2H copy of chunk k-1 overlap.
+    // chunk k and the D2H copy of chunk k-1 overlap.  The cohort kernel has no tiles: its chunks keep to ~48 MB
+    // for rows of thousands of columns too (a multiple of 16 variants).
+    const int64_t quantum = e->families ? 16 : 1024;
     int64_t cap = (int64_t)((48u << 20) / (S ? S * 24 : 24));
-    cap = std::max<int64_t>(1024, std::min<int64_t>(cap, 1 << 22)) & ~(int64_t)1023;
-    cap = std::min<int64_t>(cap, (V + 1023) & ~(int64_t)1023);
-    const bool fused = method == FS_METHOD_ES && e->is_nuclear && !e->force_generic_es; // kernel reads pl / skips single itself
+    cap = std::max<int64_t>(quantum, std::min<int64_t>(cap, 1 << 22)) & ~(quantum - 1);
+    cap = std::min<int64_t>(cap, (V + quantum - 1) & ~(quantum - 1));
+    // the kernel reads pl / skips single itself
+    const bool fused = method == FS_METHOD_ES && ((e->is_nuclear && !e->force_generic_es) || e->families);
     const bool want_single = io.single != nullptr || io.single_phred != nullptr;
     int rc = ensure_chunks(e, cap, !io.pl || !fused, io.pl != nullptr, want_single || !fused, io.phred(), io.single_phred != nullptr);
     if (rc != FS_OK) return rc;

@@ -163,17 +163,17 @@ template <class Div> __device__ __forceinline__ bool finish(Div &div, const Row3
 
 // The peeling of a nuclear family; returns true when the reference would return false.  Rows are indexed by ROLE:
 // 0 father, 1 mother, 2.. children in ped order.  wf / wm = prior * lk of the founders (the numerators of their
-// individual-only posteriors: the same products, formed once).
-template <int NC, bool X, class Div>
-__device__ __forceinline__ bool peel(const NuclearParams &P, const VariantPriors &pr, const Row3 (&L)[NC + 2], const Row3 &wf, const Row3 &wm,
-                                     const int (&col)[NC + 2], const OutRows &out, Div &div) {
-    const RunConstants &C = P.C;
+// individual-only posteriors: the same products, formed once).  male_child[c] != 0: child c is male.  Shared with the
+// cohort kernel (es_families_kernel.cu), which peels many such families per variant.
+template <int NC, bool X, class Div, class Male>
+__device__ __forceinline__ bool peel(const RunConstants &C, const Male &male_child, const VariantPriors &pr, const Row3 (&L)[NC + 2],
+                                     const Row3 &wf, const Row3 &wm, const int (&col)[NC + 2], const OutRows &out, Div &div) {
     // K[c][a][b] = sum_l (T_c[l][a][b] * lk_c[l])
     double K[NC][3][3];
 #pragma unroll
     for (int c = 0; c < NC; c++) {
         const Row3 &lc = L[2 + c];
-        const int sel = P.male_child[c] ? K_TAB_XM : K_TAB_XF;
+        const int sel = male_child[c] ? K_TAB_XM : K_TAB_XF;
 #pragma unroll
         for (int a = 0; a < 3; a++)
 #pragma unroll
@@ -221,7 +221,7 @@ __device__ __forceinline__ bool peel(const NuclearParams &P, const VariantPriors
     failed |= finish(div, pl_m, prior_m, out, col[1]);
 #pragma unroll
     for (int c = 0; c < NC; c++) {
-        const int sel = P.male_child[c] ? K_TAB_XM : K_TAB_XF;
+        const int sel = male_child[c] ? K_TAB_XM : K_TAB_XF;
         Row3 ant;
 #pragma unroll
         for (int g = 0; g < 3; g++) {
@@ -327,7 +327,7 @@ __device__ __forceinline__ bool variant_body(const NuclearParams &P, unsigned fl
         }
     }
     if (FAST) {
-        peel<NC, X>(P, pr, L, W[0], W[1], col, out, div);
+        peel<NC, X>(C, P.male_child, pr, L, W[0], W[1], col, out, div);
         *status = 0;
         // not this pass's case: an individual-only failure, a likelihood that is negative, NaN or out of the divider's range
         // (the products inherit it), the LRC gate keeping the pedigree out, another -LRC value
@@ -350,7 +350,7 @@ __device__ __forceinline__ bool variant_body(const NuclearParams &P, unsigned fl
                 out.put(col[r], p0, p1, p2);
             }
         } else {
-            failed = peel<NC, X>(P, pr, L, W[0], W[1], col, out, div);
+            failed = peel<NC, X>(C, P.male_child, pr, L, W[0], W[1], col, out, div);
         }
     }
     if (failed) { // the reference returns false: every sample of the variant is reported as NA

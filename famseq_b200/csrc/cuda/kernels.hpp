@@ -37,6 +37,26 @@ struct NuclearParams {
 // Handles B.pl (compact input, decoded through B.lut) and B.single == nullptr itself.
 cudaError_t launch_es_nuclear(const NuclearParams &P, const BatchPtrs &B, cudaStream_t stream);
 
+// ---- Elston-Stewart, cohorts of nuclear families and lone individuals (es_families_kernel.cu) ----------------
+// Families are ordered by class: [class_end[k-1], class_end[k]) have k children (k = 0: lone individuals).  The family table
+// is structure-of-arrays in device memory, F entries per array.
+constexpr int ES_FAMILIES_BLOCK = 128;
+struct FamiliesParams {
+    RunConstants C;           // C.s = S (may exceed FS_MAX_MEMBERS); C.col_male is unused, col_male below replaces it
+    int32_t n_families;
+    int32_t nc_max;           // largest sibship present (0..ES_NUCLEAR_MAX_CHILDREN)
+    int32_t group;            // threads per variant: 4, 8, 16, 32, or ES_FAMILIES_BLOCK (the whole block)
+    int32_t class_end[ES_NUCLEAR_MAX_CHILDREN + 1];
+    const int32_t *fam_col;   // [2 + ES_NUCLEAR_MAX_CHILDREN][F] input columns (-1 = unsequenced): father, mother, children in ped
+                              // order; a lone individual's column is in row 0
+    const uint8_t *fam_male;  // [F] bit c: child c is male; a lone individual: bit 0
+    const uint8_t *col_male;  // [S] gender == 1 of the member behind each input column
+};
+// Threads per variant for a row of S input columns.
+int es_families_group(int S);
+// Handles B.pl and B.single == nullptr itself, like the nuclear-family kernel.
+cudaError_t launch_es_families(const FamiliesParams &P, const BatchPtrs &B, cudaStream_t stream);
+
 // ---- Bayesian network (bn_kernel.cu) --------------------------------------------------------------
 struct BnParams {
     RunConstants C;

@@ -3,6 +3,7 @@
 
 #include <cstring>
 #include <numeric>
+#include <unordered_map>
 
 #include "../../../include/famseq_b200.h"
 
@@ -51,12 +52,15 @@ int build_pedigree(int n, const int32_t *id, const int32_t *mother_id, const int
 
     // Parent lookup scans every row without stopping, so the LAST row carrying a matching id wins
     // (family.cpp:300-316).
+    std::unordered_map<int32_t, int> row_of_id;
+    row_of_id.reserve((size_t)n);
+    for (int j = 0; j < n; j++) row_of_id[id[j]] = j;
+    auto row_of = [&](int32_t x) {
+        const auto it = row_of_id.find(x);
+        return it == row_of_id.end() ? -1 : it->second;
+    };
     for (int i = 0; i < n; i++) {
-        int m = -1, f = -1;
-        for (int j = 0; j < n; j++) {
-            if (mother_id[i] == id[j]) m = j;
-            if (father_id[i] == id[j]) f = j;
-        }
+        const int m = row_of(mother_id[i]), f = row_of(father_id[i]);
         if ((m < 0) != (f < 0)) {
             err = "This is not a fulfill family. Please check the ped file."; // family.cpp:320
             return FS_E_HALF_PARENTS;
@@ -103,11 +107,11 @@ int build_pedigree(int n, const int32_t *id, const int32_t *mother_id, const int
     // spouse--couple and child--couple.  The pedigree is peelable iff this graph is a forest.
     {
         std::vector<std::pair<int, int>> couples;
+        std::unordered_map<int64_t, int> couple_index;
         auto couple_id = [&](int m, int f) {
-            for (size_t k = 0; k < couples.size(); k++)
-                if (couples[k].first == m && couples[k].second == f) return (int)k;
-            couples.emplace_back(m, f);
-            return (int)couples.size() - 1;
+            const auto ins = couple_index.emplace((int64_t)m * n + f, (int)couples.size());
+            if (ins.second) couples.emplace_back(m, f);
+            return ins.first->second;
         };
         for (int i = 0; i < n; i++)
             if (p.mother[i] >= 0) couple_id(p.mother[i], p.father[i]);

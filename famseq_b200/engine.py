@@ -85,6 +85,10 @@ def lib() -> ctypes.CDLL:
         L.fs_create.argtypes = [P, P, ctypes.c_int, P]
         L.fs_create_multi.restype = ctypes.c_int
         L.fs_create_multi.argtypes = [P, P, P, ctypes.c_int, P]
+        L.fs_create_families.restype = ctypes.c_int
+        L.fs_create_families.argtypes = [P, P, P, ctypes.c_int, P]
+        L.fs_get_families.restype = ctypes.c_int
+        L.fs_get_families.argtypes = [P, P, P, P]
         L.fs_run_pl.restype = ctypes.c_int
         L.fs_run_pl.argtypes = [P, ctypes.c_int, I64, P, P, I32, I32, U64, I64, P, P, P, P]
         L.fs_run_pl_device.restype = ctypes.c_int
@@ -128,7 +132,8 @@ EXPORTED_SYMBOLS = ["fs_default_params", "fs_device_count", "fs_create", "fs_des
                     "fs_run_device", "fs_get_info", "fs_get_tables", "fs_alloc_pinned", "fs_free_pinned",
                     "fs_last_kernel_ms", "fs_bench_fp64_tflops", "fs_get_es_program", "fs_get_gibbs_kernel", "fs_get_es_kernel", "fs_warmup",
                     "fs_create_multi", "fs_run_pl", "fs_run_pl_device", "fs_get_pl_table",
-                    "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact"]
+                    "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact",
+                    "fs_create_families", "fs_get_families"]
 
 
 def _check(rc: int) -> None:
@@ -187,16 +192,21 @@ class Result:
 
 class Engine:
     """One pedigree compiled for one GPU (fs_create) or, with `device` a list of GPUs, for several (fs_create_multi:
-    every batch call is cut into one contiguous slice of variants per GPU)."""
+    every batch call is cut into one contiguous slice of variants per GPU).  families=True takes a cohort ped file of
+    nuclear families and lone individuals of any size (fs_create_families, Elston-Stewart only; `device` an int or a
+    list, -1 = host side only)."""
 
-    def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0):
+    def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0, families: bool = False):
         self._h = ctypes.c_void_p()
         self._keep = [_i32(ids), _i32(mother_ids), _i32(father_ids), _i32(genders), _i32(cols)]
         ped = _Pedigree(len(self._keep[0]), _ptr(self._keep[0]), _ptr(self._keep[1]), _ptr(self._keep[2]),
                         _ptr(self._keep[3]), len(self._keep[4]), _ptr(self._keep[4]))
         self.params = params if params is not None else Params.default()
         self.device = device
-        if isinstance(device, (list, tuple)):
+        if families:
+            devs = _i32(list(device) if isinstance(device, (list, tuple)) else [device])
+            _check(lib().fs_create_families(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
+        elif isinstance(device, (list, tuple)):
             devs = _i32(list(device))
             _check(lib().fs_create_multi(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
         else:
@@ -231,6 +241,15 @@ class Engine:
         mo, fa = np.zeros(self.n, np.int32), np.zeros(self.n, np.int32)
         _check(lib().fs_get_tables(self._h, _ptr(a), _ptr(xf), _ptr(xm), _ptr(mo), _ptr(fa)))
         return a, xf, xm, mo, fa
+
+    def families(self):
+        """(family[n], n_children[F]) of an engine made with families=True: the family index of each ped row (families
+        numbered by their first row) and each family's number of children (0 = a lone individual)."""
+        nf = ctypes.c_int32(0)
+        _check(lib().fs_get_families(self._h, None, ctypes.byref(nf), None))
+        fam, kids = np.zeros(self.n, np.int32), np.zeros(nf.value, np.int32)
+        _check(lib().fs_get_families(self._h, _ptr(fam), None, _ptr(kids)))
+        return fam, kids
 
     def es_program(self):
         """(words, n_slots) of the compiled Elston-Stewart message program (introspection, see es_program.hpp)."""

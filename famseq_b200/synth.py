@@ -268,6 +268,15 @@ def forest(families, shuffle_seed=None):
     return ped, [np.nonzero(fam == f)[0] for f in range(len(families))]
 
 
+def cohort(n_trios: int, n_quads: int = 0, n_sibships_3to5: int = 0, n_lone: int = 0, seed: int = 0, shuffle: bool = False):
+    """A cohort ped file (`forest`): trios, quads, sibships of 3..5 children (sizes drawn from `seed`) and lone
+    individuals, in that order, or with their rows interleaved at random when `shuffle`."""
+    rng = np.random.default_rng(seed)
+    fams = [sibship(1)] * n_trios + [sibship(2)] * n_quads + [sibship(int(k)) for k in rng.integers(3, 6, n_sibships_3to5)]
+    fams += [_mk([(1, 0, 0, 1 + k % 2)]) for k in range(n_lone)]
+    return forest(fams, shuffle_seed=int(rng.integers(1 << 30)) if shuffle else None)
+
+
 PEDIGREES = {"trio": trio, "ped14": ped14, "ped40": ped40, "half_sibs": half_sibs, "three_wives": three_wives, "ped100": ped100,
              "cousins_loop": cousins_loop}
 

@@ -102,6 +102,18 @@ void fs_destroy(fs_engine *e);
  * The *_device entry points need a single-GPU engine (FS_E_ARG otherwise). */
 int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
 
+/* A ped file of many unrelated families (a cohort), for Elston-Stewart.  The pedigree is split into its connected
+ * families; each must be a lone individual or a nuclear family (two founders, 1..5 childless children of both, any
+ * member unsequenced).  No limit on the total member count beyond memory.  Same validation and error codes as fs_create
+ * for the ped rows themselves; a family of another shape is refused with FS_E_TOO_LARGE, the message naming its first ped
+ * id.  Outputs are those of the reference peeling the whole file as one family: per-variant LRC gate and failure over all
+ * samples.  ES only: BN / MCMC runs fail with FS_E_TOO_LARGE.  ndev == 1 gives a single-GPU engine (the *_device entry
+ * points work, device -1 = host only); ndev > 1 slices batches like fs_create_multi. */
+int fs_create_families(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
+/* family[n]: family index of each ped row (families numbered by their first row); n_children[*n_families]: 0 for a lone
+ * individual.  Either pointer may be NULL.  FS_E_ARG on an engine that fs_create made. */
+int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children);
+
 /* Thread-local text of the last error raised on the calling thread. */
 const char *fs_last_error(void);
 
