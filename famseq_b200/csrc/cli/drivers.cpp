@@ -290,8 +290,8 @@ struct Engine {
             fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
         fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), (int32_t)cm.engine_cols.size(),
                        cm.engine_cols.data()};
-        // ped files past the 128 members of one pedigree: a cohort of nuclear families and lone individuals (ES only)
-        const int rc = id.size() > kMaxPedigreeMembers ? fs_create_families(&fp, &prm, devices.data(), (int)devices.size(), &h)
+        // ped files past the 128 members of one pedigree: a cohort of loop-free families (ES only)
+        const int rc = id.size() > kMaxPedigreeMembers ? fs_create_cohort(&fp, &prm, devices.data(), (int)devices.size(), &h)
                                                        : fs_create_multi(&fp, &prm, devices.data(), (int)devices.size(), &h);
         if (rc != FS_OK) {
             std::cout << fs_last_error() << std::endl;
@@ -749,7 +749,7 @@ bool check_family(const PedRows &ped) {
     fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), 0, nullptr};
     fs_engine *h = nullptr;
     const int host_only = -1;
-    const int rc = id.size() > kMaxPedigreeMembers ? fs_create_families(&fp, nullptr, &host_only, 1, &h) : fs_create(&fp, nullptr, -1, &h);
+    const int rc = id.size() > kMaxPedigreeMembers ? fs_create_cohort(&fp, nullptr, &host_only, 1, &h) : fs_create(&fp, nullptr, -1, &h);
     fs_destroy(h);
     if (rc == FS_OK) return true;
     if (rc == FS_E_GENDER)

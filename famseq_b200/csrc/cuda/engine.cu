@@ -114,6 +114,15 @@ struct GibbsJitState {
     double pilot_serial_fraction = -1; // what the pilot measured (fs_get_info reports the generator)
     unsigned long long *d_vote_stats = nullptr;
 };
+// Uploads `v` to a new device array (nothing for an empty vector).
+template <class T> cudaError_t upload(const std::vector<T> &v, const T **dst) {
+    if (v.empty()) return cudaSuccess;
+    T *d = nullptr;
+    cudaError_t rc = cudaMalloc(&d, v.size() * sizeof(T));
+    if (rc != cudaSuccess) return rc;
+    *dst = d;
+    return cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+}
 } // namespace
 
 struct fs_engine {
@@ -159,10 +168,12 @@ struct fs_engine {
 
     std::vector<fs_engine *> parts; // fs_create_multi: one single-device engine per GPU (this one then has device -1)
 
-    // fs_create_families: a cohort of nuclear families and lone individuals, ES only (es_families_kernel.cu)
+    // fs_create_families: a cohort of nuclear families and lone individuals, ES only (es_families_kernel.cu);
+    // fs_create_cohort: families of any loop-free shape too, through per-family message programs (es_cohort_kernel.cu)
     bool families = false;
     FamilyTable fam_table;
     FamiliesParams fam; // its device arrays are owned by this engine
+    CohortParams cohort; // fs_create_cohort with program families (cohort.n_pf > 0); its device arrays are owned too
 };
 
 extern "C" {
@@ -244,13 +255,17 @@ void fs_destroy(fs_engine *e) {
         cudaFree(const_cast<int32_t *>(e->fam.fam_col));
         cudaFree(const_cast<uint8_t *>(e->fam.fam_male));
         cudaFree(const_cast<uint8_t *>(e->fam.col_male));
+        cudaFree(const_cast<uint32_t *>(e->cohort.words));
+        for (const int32_t *a : {e->cohort.prog_off, e->cohort.prog_slots, e->cohort.prog_cols, e->cohort.pf_prog, e->cohort.pf_col_off, e->cohort.cols})
+            cudaFree(const_cast<int32_t *>(a));
     }
     delete e;
 }
 
-// fs_create (families == false) and fs_create_families on one device (-1: host side only).
-static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, fs_engine **out) {
-    if (!ped || !out) return fail(FS_E_ARG, families ? "fs_create_families: null argument" : "fs_create: null argument");
+// fs_create (families == false), fs_create_families and (any_shape) fs_create_cohort on one device (-1: host side only).
+static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, bool any_shape, fs_engine **out) {
+    const char *who = any_shape ? "fs_create_cohort" : families ? "fs_create_families" : "fs_create";
+    if (!ped || !out) return fail(FS_E_ARG, std::string(who) + ": null argument");
     *out = nullptr;
     fs_params prm;
     if (params)
@@ -307,7 +322,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
     e->pl_table.resize(FS_PL_TABLE_SIZE);
     for (int k = 0; k < FS_PL_TABLE_SIZE; k++) e->pl_table[k] = std::pow(10.0, -std::fabs((double)k) / 10.0);
     if (families) {
-        rc = build_families(e->ped, ped->id, e->fam_table, err);
+        rc = build_families(e->ped, ped->id, e->fam_table, err, any_shape);
         if (rc != FS_OK) {
             delete e;
             return fail(rc, err);
@@ -315,7 +330,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
         e->families = true;
         const FamilyTable &t = e->fam_table;
         e->fam.C = C;
-        e->fam.n_families = t.n_families();
+        e->fam.n_families = t.n_peeled;
         e->fam.nc_max = t.nc_max;
         e->fam.group = es_families_group(C.s);
         std::memcpy(e->fam.class_end, t.class_end, sizeof t.class_end);
@@ -420,9 +435,40 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
             if (crc == cudaSuccess) e->fam.col_male = d_col_male, crc = cudaMemcpy(d_col, t.col.data(), t.col.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
             if (crc == cudaSuccess) crc = cudaMemcpy(d_male, t.male.data(), t.male.size(), cudaMemcpyHostToDevice);
             if (crc == cudaSuccess) crc = cudaMemcpy(d_col_male, col_male.data(), col_male.size(), cudaMemcpyHostToDevice);
+            if (crc == cudaSuccess && !t.pf_order.empty()) { // the program families
+                CohortParams &P = e->cohort;
+                P.fam = e->fam;
+                P.n_pf = (int32_t)t.pf_order.size();
+                P.max_vectors = t.max_vectors;
+                // block size: es_pick_block's rule for the largest vector file of any program
+                auto largest = std::make_unique<EsParams>();
+                largest->C.s = t.max_vectors;
+                P.tb = es_pick_block(*largest, e->smem_limit);
+                if (P.tb == 0) {
+                    int q = 0;
+                    for (int k = 1; k < t.n_programs(); k++)
+                        if (t.prog_cols[k] + t.prog_slots[k] > t.prog_cols[q] + t.prog_slots[q]) q = k;
+                    const int32_t first_id = ped->id[std::find(t.family_of.begin(), t.family_of.end(), t.prog_family[q]) - t.family_of.begin()];
+                    fs_destroy(e);
+                    return fail(FS_E_TOO_LARGE, "ped file family of " + std::to_string(first_id) +
+                                                    ": pedigree too large for the ES kernel: message scratch exceeds shared memory");
+                }
+                std::vector<int32_t> pf_prog, pf_col_off;
+                for (int f : t.pf_order) {
+                    pf_prog.push_back(t.program[f]);
+                    pf_col_off.push_back(t.col_off[f]);
+                }
+                crc = upload(t.words, &P.words);
+                if (crc == cudaSuccess) crc = upload(t.prog_off, &P.prog_off);
+                if (crc == cudaSuccess) crc = upload(t.prog_slots, &P.prog_slots);
+                if (crc == cudaSuccess) crc = upload(t.prog_cols, &P.prog_cols);
+                if (crc == cudaSuccess) crc = upload(pf_prog, &P.pf_prog);
+                if (crc == cudaSuccess) crc = upload(pf_col_off, &P.pf_col_off);
+                if (crc == cudaSuccess) crc = upload(t.cols, &P.cols);
+            }
             if (crc != cudaSuccess) {
                 fs_destroy(e); // releases what was allocated
-                return cuda_fail(crc, "fs_create_families: family table upload");
+                return cuda_fail(crc, (std::string(who) + ": family table upload").c_str());
             }
         }
     }
@@ -431,24 +477,25 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
 }
 
 int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_engine **out) {
-    return create_engine(ped, params, device, false, out);
+    return create_engine(ped, params, device, false, false, out);
 }
 
-static int create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, bool families, fs_engine **out) {
-    const char *who = families ? "fs_create_families" : "fs_create_multi";
+static int create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, bool families, bool any_shape,
+                        fs_engine **out) {
+    const char *who = any_shape ? "fs_create_cohort" : families ? "fs_create_families" : "fs_create_multi";
     if (!ped || !out || !devices || ndev < 1) return fail(FS_E_ARG, std::string(who) + ": null argument or no device");
     *out = nullptr;
     // a device may be listed more than once: every entry gets its own pipeline (streams, buffers) on that GPU
     for (int g = 0; g < ndev; g++)
         if (devices[g] < 0 && !(families && ndev == 1)) return fail(FS_E_ARG, std::string(who) + ": negative device");
-    if (ndev == 1) return create_engine(ped, params, devices[0], families, out);
+    if (ndev == 1) return create_engine(ped, params, devices[0], families, any_shape, out);
     // the front engine holds the host side (pedigree, tables, info); the parts own the GPUs
     fs_engine *front = nullptr;
-    int rc = create_engine(ped, params, -1, families, &front);
+    int rc = create_engine(ped, params, -1, families, any_shape, &front);
     if (rc != FS_OK) return rc;
     for (int g = 0; g < ndev; g++) {
         fs_engine *part = nullptr;
-        rc = create_engine(ped, params, devices[g], families, &part);
+        rc = create_engine(ped, params, devices[g], families, any_shape, &part);
         if (rc != FS_OK) {
             const std::string keep = g_last_error;
             fs_destroy(front);
@@ -461,20 +508,45 @@ static int create_multi(const fs_pedigree *ped, const fs_params *params, const i
 }
 
 int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    return create_multi(ped, params, devices, ndev, false, out);
+    return create_multi(ped, params, devices, ndev, false, false, out);
 }
 
 int fs_create_families(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    return create_multi(ped, params, devices, ndev, true, out);
+    return create_multi(ped, params, devices, ndev, true, false, out);
+}
+
+int fs_create_cohort(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
+    return create_multi(ped, params, devices, ndev, true, true, out);
 }
 
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children) {
     if (!e) return fail(FS_E_ARG, "fs_get_families: null engine");
-    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families");
+    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families or fs_create_cohort");
     const FamilyTable &t = e->fam_table;
     if (family) std::memcpy(family, t.family_of.data(), t.family_of.size() * sizeof(int32_t));
     if (n_families) *n_families = t.n_families();
     if (n_children) std::memcpy(n_children, t.n_children.data(), t.n_children.size() * sizeof(int32_t));
+    return FS_OK;
+}
+
+int fs_get_family_program(const fs_engine *e, int32_t f, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
+                          int32_t *cols, int32_t *n_cols, int32_t *program) {
+    if (!e) return fail(FS_E_ARG, "fs_get_family_program: null engine");
+    if (!e->families) return fail(FS_E_ARG, "fs_get_family_program: the engine was not made by fs_create_families or fs_create_cohort");
+    const FamilyTable &t = e->fam_table;
+    if (f < 0 || f >= t.n_families()) return fail(FS_E_ARG, "fs_get_family_program: no family " + std::to_string(f));
+    const int q = t.program.empty() ? -1 : t.program[f];
+    const int nw = q < 0 ? 0 : (q + 1 < t.n_programs() ? t.prog_off[q + 1] : (int)t.words.size()) - t.prog_off[q];
+    const int nc = q < 0 ? 0 : t.prog_cols[q];
+    if (program) *program = q;
+    if (n_words) *n_words = nw;
+    if (n_slots) *n_slots = q < 0 ? 0 : t.prog_slots[q];
+    if (n_cols) *n_cols = nc;
+    if (words && nw) {
+        if (capacity < nw) return fail(FS_E_ARG, "fs_get_family_program: buffer too small");
+        std::memcpy(words, t.words.data() + t.prog_off[q], sizeof(uint32_t) * (size_t)nw);
+    }
+    if (cols && nc) std::memcpy(cols, t.cols.data() + t.col_off[f], sizeof(int32_t) * (size_t)nc);
     return FS_OK;
 }
 
@@ -741,6 +813,11 @@ static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t
         const int rc = ensure_pl_table(e, stream);
         if (rc != FS_OK) return rc;
         B.lut = e->d_pl_table;
+    }
+    if (method == FS_METHOD_ES && e->families && e->cohort.n_pf > 0) {
+        FS_CUDA(launch_es_cohort(e->cohort, B, stream));
+        e->launches += 3;
+        return FS_OK;
     }
     if (method == FS_METHOD_ES && e->families) {
         FS_CUDA(launch_es_families(e->fam, B, stream));

@@ -57,6 +57,28 @@ int es_families_group(int S);
 // Handles B.pl and B.single == nullptr itself, like the nuclear-family kernel.
 cudaError_t launch_es_families(const FamiliesParams &P, const BatchPtrs &B, cudaStream_t stream);
 
+// ---- Elston-Stewart, cohorts with families of any loop-free shape (es_cohort_kernel.cu) ------------------------
+// The families es_families_kernel takes are peeled as there; every other family runs its deduplicated message program
+// (host/families.hpp), one block per (variant tile, family).  The program arrays live in device memory.
+struct CohortParams {
+    FamiliesParams fam;         // the column pass, the nuclear families and lone individuals
+    int32_t n_pf;               // families peeled by a program
+    int32_t tb;                 // variants per block of the program kernel: 128, 64 or 32
+    int32_t max_vectors;        // largest local columns + scratch vectors of any program: sizes the vector file
+    const uint32_t *words;      // concatenated programs
+    const int32_t *prog_off;    // [P] word offset of each program
+    const int32_t *prog_slots;  // [P] scratch vectors
+    const int32_t *prog_cols;   // [P] local columns
+    const int32_t *pf_prog;     // [n_pf] program of each program family, sorted by program
+    const int32_t *pf_col_off;  // [n_pf] offset of its local -> global column map in `cols`
+    const int32_t *cols;        // concatenated column maps
+};
+// Shared memory of the program kernel's vector file at block size tb.
+size_t es_cohort_smem_bytes(int max_vectors, int tb);
+// Three launches whatever the number of families: the column pass and nuclear families, the programs, the failure rule.
+// Handles B.pl and B.single == nullptr itself.
+cudaError_t launch_es_cohort(const CohortParams &P, const BatchPtrs &B, cudaStream_t stream);
+
 // ---- Bayesian network (bn_kernel.cu) --------------------------------------------------------------
 struct BnParams {
     RunConstants C;

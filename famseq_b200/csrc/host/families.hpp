@@ -1,6 +1,7 @@
 // families.hpp -- a ped file of many unrelated families (a cohort) split into its connected families for the
-// cohort Elston-Stewart kernel (cuda/es_families_kernel.cu).  Each family must be a lone individual or a nuclear family:
-// two founders and 1..5 childless children of both.
+// cohort Elston-Stewart kernels.  Lone individuals and nuclear families (two founders and 1..5 childless children of both)
+// are peeled by cuda/es_families_kernel.cu; with `any_shape`, every other loop-free family of at most 128 members gets an
+// ES message program of its own (host/es_program.cpp), run by cuda/es_cohort_kernel.cu.
 #pragma once
 
 #include <cstdint>
@@ -15,18 +16,34 @@ constexpr int FAMILY_MAX_CHILDREN = 5;
 
 struct FamilyTable {
     std::vector<int32_t> family_of;  // [n] family of each ped row; families are numbered by their first row
-    std::vector<int32_t> n_children; // [F] 0 for a lone individual
-    // Device order: families sorted by number of children (stable), structure-of-arrays.
-    std::vector<int32_t> col;         // [2 + FAMILY_MAX_CHILDREN][F] input columns (-1 = unsequenced): father, mother,
+    std::vector<int32_t> n_children; // [F] 0 for a lone individual; a program family: its non-founder members
+    // Device order of the families the nuclear kernel peels: sorted by number of children (stable), structure-of-arrays.
+    std::vector<int32_t> col;         // [2 + FAMILY_MAX_CHILDREN][n_peeled] input columns (-1 = unsequenced): father, mother,
                                       // children in ped order; a lone individual's column is in row 0
-    std::vector<uint8_t> male;        // [F] bit c: child c is male; a lone individual: bit 0
+    std::vector<uint8_t> male;        // [n_peeled] bit c: child c is male; a lone individual: bit 0
     int32_t class_end[FAMILY_MAX_CHILDREN + 1] = {}; // device-order families [class_end[k-1], class_end[k]) have k children
     int32_t nc_max = 0;
+    int32_t n_peeled = 0;             // families of the nuclear kernel (all of them without any_shape)
+
+    // Program families (any_shape only).  Programs are deduplicated by (words, n_slots); their operands index the
+    // family's own vector file: local columns (its sequenced members in increasing global input column), scratch, priors,
+    // ones -- nothing depends on the cohort's column count.
+    std::vector<int32_t> program;     // [F] program of each family, -1 for a family of the nuclear kernel
+    std::vector<int32_t> col_off;     // [F] offset of the family's local -> global column map in `cols`, -1 likewise
+    std::vector<int32_t> cols;        // concatenated column maps
+    std::vector<uint32_t> words;      // concatenated programs
+    std::vector<int32_t> prog_off, prog_slots, prog_cols; // [P] word offset, scratch vectors, local columns
+    std::vector<int32_t> prog_family; // [P] first family that runs the program (names it in messages)
+    std::vector<int32_t> pf_order;    // program families sorted by program, then family: the device order
+    int32_t max_vectors = 0;          // largest local columns + scratch vectors of any program
+
     int n_families() const { return (int)n_children.size(); }
+    int n_programs() const { return (int)prog_off.size(); }
 };
 
-// FS_OK, or FS_E_TOO_LARGE with a message naming the first ped id of the first family of another shape.  Linear in the
-// number of ped rows.
-int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err);
+// FS_OK, or an error with a message naming the first ped id of the first family that is refused: FS_E_TOO_LARGE for a
+// family of another shape (without any_shape) or over a limit of the ES message program, FS_E_LOOP for a looped family
+// (any_shape).  Linear in the number of ped rows plus the compile time of the program families.
+int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err, bool any_shape = false);
 
 } // namespace famseq

@@ -89,6 +89,10 @@ def lib() -> ctypes.CDLL:
         L.fs_create_families.argtypes = [P, P, P, ctypes.c_int, P]
         L.fs_get_families.restype = ctypes.c_int
         L.fs_get_families.argtypes = [P, P, P, P]
+        L.fs_create_cohort.restype = ctypes.c_int
+        L.fs_create_cohort.argtypes = [P, P, P, ctypes.c_int, P]
+        L.fs_get_family_program.restype = ctypes.c_int
+        L.fs_get_family_program.argtypes = [P, I32, P, I32, P, P, P, P, P]
         L.fs_run_pl.restype = ctypes.c_int
         L.fs_run_pl.argtypes = [P, ctypes.c_int, I64, P, P, I32, I32, U64, I64, P, P, P, P]
         L.fs_run_pl_device.restype = ctypes.c_int
@@ -133,7 +137,7 @@ EXPORTED_SYMBOLS = ["fs_default_params", "fs_device_count", "fs_create", "fs_des
                     "fs_last_kernel_ms", "fs_bench_fp64_tflops", "fs_get_es_program", "fs_get_gibbs_kernel", "fs_get_es_kernel", "fs_warmup",
                     "fs_create_multi", "fs_run_pl", "fs_run_pl_device", "fs_get_pl_table",
                     "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact",
-                    "fs_create_families", "fs_get_families"]
+                    "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program"]
 
 
 def _check(rc: int) -> None:
@@ -194,18 +198,21 @@ class Engine:
     """One pedigree compiled for one GPU (fs_create) or, with `device` a list of GPUs, for several (fs_create_multi:
     every batch call is cut into one contiguous slice of variants per GPU).  families=True takes a cohort ped file of
     nuclear families and lone individuals of any size (fs_create_families, Elston-Stewart only; `device` an int or a
-    list, -1 = host side only)."""
+    list, -1 = host side only); cohort=True takes one whose families may also have any other loop-free shape
+    (fs_create_cohort, same rules)."""
 
-    def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0, families: bool = False):
+    def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0, families: bool = False,
+                 cohort: bool = False):
         self._h = ctypes.c_void_p()
         self._keep = [_i32(ids), _i32(mother_ids), _i32(father_ids), _i32(genders), _i32(cols)]
         ped = _Pedigree(len(self._keep[0]), _ptr(self._keep[0]), _ptr(self._keep[1]), _ptr(self._keep[2]),
                         _ptr(self._keep[3]), len(self._keep[4]), _ptr(self._keep[4]))
         self.params = params if params is not None else Params.default()
         self.device = device
-        if families:
+        if families or cohort:
             devs = _i32(list(device) if isinstance(device, (list, tuple)) else [device])
-            _check(lib().fs_create_families(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
+            create = lib().fs_create_cohort if cohort else lib().fs_create_families
+            _check(create(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
         elif isinstance(device, (list, tuple)):
             devs = _i32(list(device))
             _check(lib().fs_create_multi(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
@@ -243,13 +250,24 @@ class Engine:
         return a, xf, xm, mo, fa
 
     def families(self):
-        """(family[n], n_children[F]) of an engine made with families=True: the family index of each ped row (families
-        numbered by their first row) and each family's number of children (0 = a lone individual)."""
+        """(family[n], n_children[F]) of an engine made with families=True or cohort=True: the family index of each ped row
+        (families numbered by their first row) and each family's number of children (0 = a lone individual; the
+        non-founder members of a family peeled by a message program)."""
         nf = ctypes.c_int32(0)
         _check(lib().fs_get_families(self._h, None, ctypes.byref(nf), None))
         fam, kids = np.zeros(self.n, np.int32), np.zeros(nf.value, np.int32)
         _check(lib().fs_get_families(self._h, _ptr(fam), None, _ptr(kids)))
         return fam, kids
+
+    def family_program(self, f: int):
+        """(words, n_slots, cols, program) of family f of a cohort=True engine: the message program it runs, the global input
+        column of each of its local columns, and the program's index (-1 and empty arrays: the nuclear kernel peels it)."""
+        n_words, n_slots, n_cols, prog = ctypes.c_int32(0), ctypes.c_int32(0), ctypes.c_int32(0), ctypes.c_int32(0)
+        _check(lib().fs_get_family_program(self._h, f, None, 0, ctypes.byref(n_words), ctypes.byref(n_slots), None,
+                                           ctypes.byref(n_cols), ctypes.byref(prog)))
+        words, cols = np.zeros(n_words.value, np.uint32), np.zeros(n_cols.value, np.int32)
+        _check(lib().fs_get_family_program(self._h, f, _ptr(words), n_words.value, None, None, _ptr(cols), None, None))
+        return words, int(n_slots.value), cols, int(prog.value)
 
     def es_program(self):
         """(words, n_slots) of the compiled Elston-Stewart message program (introspection, see es_program.hpp)."""

@@ -110,9 +110,26 @@ int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *
  * samples.  ES only: BN / MCMC runs fail with FS_E_TOO_LARGE.  ndev == 1 gives a single-GPU engine (the *_device entry
  * points work, device -1 = host only); ndev > 1 slices batches like fs_create_multi. */
 int fs_create_families(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
+/* The same for cohorts whose families may have any shape: three generations, half-sibs, several spouses, sibships of six
+ * or more.  Lone individuals and nuclear families (1..5 children) are peeled as by fs_create_families; every other family
+ * is accepted when fs_create would run Elston-Stewart on it as a pedigree of its own (at most 128 members, no loop, a
+ * message program within ES_MAX_WORDS and, on a device, a vector file that fits shared memory) and is peeled by its own
+ * message program, compiled on its rows in file order with its sequenced members as columns in increasing input column.
+ * Families of one shape and one sequencing pattern share one program.  Refusals name the family's first ped id
+ * ("ped file family of <id>: ..."): FS_E_LOOP for a looped family, FS_E_TOO_LARGE for one over a limit.  Ped-row
+ * validation, error codes, the whole-file LRC gate and failure rule, ES only and the device slicing are those of
+ * fs_create_families.  A batch is three kernel launches (one without program families), whatever the number of families. */
+int fs_create_cohort(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
 /* family[n]: family index of each ped row (families numbered by their first row); n_children[*n_families]: 0 for a lone
- * individual.  Either pointer may be NULL.  FS_E_ARG on an engine that fs_create made. */
+ * individual, the number of non-founder members for a family peeled by a program (fs_create_cohort).  Either pointer may
+ * be NULL.  FS_E_ARG on an engine that fs_create made. */
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children);
+/* Family f of an fs_create_cohort engine (numbered as in fs_get_families): the deduplicated message program it runs
+ * (words: capacity in words; *n_words, *n_slots as fs_get_es_program), cols[*n_cols]: the global input column of each of
+ * its local columns, *program: the program's index, or -1 for a family the nuclear kernel peels (then *n_words = 0 and
+ * *n_cols = 0).  Every pointer may be NULL.  Introspection: tests interpret the programs on the CPU. */
+int fs_get_family_program(const fs_engine *e, int32_t f, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
+                          int32_t *cols, int32_t *n_cols, int32_t *program);
 
 /* Thread-local text of the last error raised on the calling thread. */
 const char *fs_last_error(void);
