@@ -17,8 +17,9 @@ struct PedRows { // the five ped columns, file.cpp:24-62
 bool read_ped(const std::string &path, PedRows &out);
 
 // Checks the pedigree the way family::init does (half-specified parents, parent genders) before any output
-// is written.  Prints the reference's messages; false = fatal.
-bool check_family(const PedRows &ped);
+// is written.  Prints the reference's messages; false = fatal.  family_bn (-familyBN -method 1): the ped file is checked
+// as the cohort Bayesian-network engine takes it (every family on its own, loops allowed).
+bool check_family(const PedRows &ped, bool family_bn);
 
 bool run_vcf(const VcfOptions &opt, const PedRows &ped);
 bool run_lk(const LkOptions &opt, const PedRows &ped);

@@ -66,6 +66,7 @@ static void help() {
         {"-l\t\t", "File of tab-separated 'chromosome position' lines; only these positions are processed (vcf mode)."},
         {"-device\t\t", "(this implementation) CUDA device to run on. The default is 0."},
         {"-seed\t\t", "(this implementation) Seed of the counter-based random number generator of the MCMC method. The default is 1."},
+        {"-familyBN\t", "(this implementation) With -method 1: compute the Bayesian network of each family of the ped file on its own, for ped files of any size and families with loops (at most 31 members each). Members' posteriors equal those of the whole-file network except where its product of all members' probabilities leaves the double range."},
     };
     for (auto &r : rows) cout << r[0] << r[1] << endl << endl;
 }
@@ -102,7 +103,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set family." << endl;
             return -1;
         }
-        if (!check_family(ped)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1)) {
             cout << "Cannot set family." << endl;
             return -1;
         }
@@ -123,7 +124,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set Family." << endl;
             return -1;
         }
-        if (!check_family(ped)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1)) {
             cout << "Cannot set Family." << endl;
             return -1;
         }

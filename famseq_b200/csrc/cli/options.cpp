@@ -137,6 +137,10 @@ int common_option(Scanner &sc, const std::string &opt, CommonOptions &o) {
         o.device = (o.devices.empty() || o.devices[0] < 0) ? 0 : o.devices[0];
         return 1;
     }
+    if (opt == "familyBN") {
+        o.family_bn = true;
+        return 1;
+    }
     if (opt == "seed" && sc.value_follows()) {
         o.seed = std::strtoull(sc.take(), nullptr, 10);
         return 1;

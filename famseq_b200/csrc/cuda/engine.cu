@@ -174,6 +174,9 @@ struct fs_engine {
     FamilyTable fam_table;
     FamiliesParams fam; // its device arrays are owned by this engine
     CohortParams cohort; // fs_create_cohort with program families (cohort.n_pf > 0); its device arrays are owned too
+    // fs_create_cohort_bn: every family enumerated on its own (bn_cohort_kernel.cu), BN only; its device arrays are owned too
+    bool cohort_bn = false;
+    BnCohortParams bn_cohort;
 };
 
 extern "C" {
@@ -258,13 +261,21 @@ void fs_destroy(fs_engine *e) {
         cudaFree(const_cast<uint32_t *>(e->cohort.words));
         for (const int32_t *a : {e->cohort.prog_off, e->cohort.prog_slots, e->cohort.prog_cols, e->cohort.pf_prog, e->cohort.pf_col_off, e->cohort.cols})
             cudaFree(const_cast<int32_t *>(a));
+        cudaFree(const_cast<BnPlan *>(e->bn_cohort.plans));
+        for (const int32_t *a : {e->bn_cohort.fam_plan, e->bn_cohort.fam_col_off, e->bn_cohort.cols}) cudaFree(const_cast<int32_t *>(a));
     }
     delete e;
 }
 
-// fs_create (families == false), fs_create_families and (any_shape) fs_create_cohort on one device (-1: host side only).
-static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, bool any_shape, fs_engine **out) {
-    const char *who = any_shape ? "fs_create_cohort" : families ? "fs_create_families" : "fs_create";
+static const char *creator(bool families, FamilyMode mode) {
+    if (!families) return "fs_create";
+    return mode == FamilyMode::BN ? "fs_create_cohort_bn" : mode == FamilyMode::ANY_SHAPE ? "fs_create_cohort" : "fs_create_families";
+}
+
+// fs_create (families == false), and with families == true fs_create_families, fs_create_cohort or fs_create_cohort_bn by
+// `mode`, on one device (-1: host side only).
+static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, FamilyMode mode, fs_engine **out) {
+    const char *who = creator(families, mode);
     if (!ped || !out) return fail(FS_E_ARG, std::string(who) + ": null argument");
     *out = nullptr;
     fs_params prm;
@@ -322,7 +333,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
     e->pl_table.resize(FS_PL_TABLE_SIZE);
     for (int k = 0; k < FS_PL_TABLE_SIZE; k++) e->pl_table[k] = std::pow(10.0, -std::fabs((double)k) / 10.0);
     if (families) {
-        rc = build_families(e->ped, ped->id, e->fam_table, err, any_shape);
+        rc = build_families(e->ped, ped->id, e->fam_table, err, mode);
         if (rc != FS_OK) {
             delete e;
             return fail(rc, err);
@@ -338,6 +349,19 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
         e->bn_err = e->mcmc_err = "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(t.n_families()) +
                                   " families: only Elston-Stewart (-method 2) runs on ped files over " +
                                   std::to_string(FS_MAX_MEMBERS) + " members";
+        if (mode == FamilyMode::BN) {
+            e->cohort_bn = true;
+            e->bn_rc = FS_OK;
+            e->es_rc = e->mcmc_rc = FS_E_ARG;
+            e->es_err = e->mcmc_err = "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(t.n_families()) +
+                                      " families: this engine runs the Bayesian network (-method 1) only; Elston-Stewart on "
+                                      "cohorts is fs_create_cohort";
+            // fs_get_info: the largest family's plan
+            int big = 0;
+            for (int q = 1; q < (int)t.plans.size(); q++)
+                if (t.plans[q].n_levels > t.plans[big].n_levels) big = q;
+            if (!t.plans.empty()) e->bn.plan = t.plans[big];
+        }
     }
 
     // ---- pedigree compilers ----------------------------------------------------------------------
@@ -412,7 +436,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
                 e->es_err = "pedigree too large for the ES kernel: message scratch exceeds shared memory";
             }
         }
-        if (e->bn_rc == FS_OK && bn_smem_bytes(e->bn) > e->smem_limit) {
+        if (e->bn_rc == FS_OK && !families && bn_smem_bytes(e->bn) > e->smem_limit) {
             e->bn_rc = FS_E_TOO_LARGE;
             e->bn_err = "pedigree too large for the BN kernel: per-thread odometer state exceeds shared memory";
         }
@@ -466,6 +490,32 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
                 if (crc == cudaSuccess) crc = upload(pf_col_off, &P.pf_col_off);
                 if (crc == cudaSuccess) crc = upload(t.cols, &P.cols);
             }
+            if (crc == cudaSuccess && e->cohort_bn) { // the plans, the column maps and the launch classes
+                BnCohortParams &P = e->bn_cohort;
+                P.head = e->fam;
+                for (size_t q = 0; q < t.plans.size(); q++)
+                    if (bn_cohort_smem_bytes(t.plans[q]) + sizeof(BnPlan) > e->smem_limit) {
+                        const int32_t first_id = ped->id[std::find(t.family_of.begin(), t.family_of.end(), t.plan_family[q]) - t.family_of.begin()];
+                        fs_destroy(e);
+                        return fail(FS_E_TOO_LARGE, "ped file family of " + std::to_string(first_id) +
+                                                        ": pedigree too large for the BN kernel: per-thread odometer state exceeds shared memory");
+                    }
+                std::vector<int32_t> fam_plan, fam_col_off;
+                for (int f : t.bn_order) {
+                    fam_plan.push_back(t.plan[f]);
+                    fam_col_off.push_back(t.col_off[f]);
+                }
+                for (size_t k = 0, d = 0; k < t.bn_class_end.size(); k++) {
+                    const BnPlan &first = t.plans[fam_plan[d]];
+                    BnCohortClass c{first.u, first.independent, first.factor_leaves, first.group, (int32_t)d, t.bn_class_end[k], 0};
+                    for (; (int32_t)d < c.end; d++) c.smem = std::max(c.smem, bn_cohort_smem_bytes(t.plans[fam_plan[d]]));
+                    P.classes.push_back(c);
+                }
+                crc = upload(t.plans, &P.plans);
+                if (crc == cudaSuccess) crc = upload(fam_plan, &P.fam_plan);
+                if (crc == cudaSuccess) crc = upload(fam_col_off, &P.fam_col_off);
+                if (crc == cudaSuccess) crc = upload(t.cols, &P.cols);
+            }
             if (crc != cudaSuccess) {
                 fs_destroy(e); // releases what was allocated
                 return cuda_fail(crc, (std::string(who) + ": family table upload").c_str());
@@ -477,25 +527,25 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
 }
 
 int fs_create(const fs_pedigree *ped, const fs_params *params, int device, fs_engine **out) {
-    return create_engine(ped, params, device, false, false, out);
+    return create_engine(ped, params, device, false, FamilyMode::NUCLEAR, out);
 }
 
-static int create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, bool families, bool any_shape,
+static int create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, bool families, FamilyMode mode,
                         fs_engine **out) {
-    const char *who = any_shape ? "fs_create_cohort" : families ? "fs_create_families" : "fs_create_multi";
+    const char *who = families ? creator(families, mode) : "fs_create_multi";
     if (!ped || !out || !devices || ndev < 1) return fail(FS_E_ARG, std::string(who) + ": null argument or no device");
     *out = nullptr;
     // a device may be listed more than once: every entry gets its own pipeline (streams, buffers) on that GPU
     for (int g = 0; g < ndev; g++)
         if (devices[g] < 0 && !(families && ndev == 1)) return fail(FS_E_ARG, std::string(who) + ": negative device");
-    if (ndev == 1) return create_engine(ped, params, devices[0], families, any_shape, out);
+    if (ndev == 1) return create_engine(ped, params, devices[0], families, mode, out);
     // the front engine holds the host side (pedigree, tables, info); the parts own the GPUs
     fs_engine *front = nullptr;
-    int rc = create_engine(ped, params, -1, families, any_shape, &front);
+    int rc = create_engine(ped, params, -1, families, mode, &front);
     if (rc != FS_OK) return rc;
     for (int g = 0; g < ndev; g++) {
         fs_engine *part = nullptr;
-        rc = create_engine(ped, params, devices[g], families, any_shape, &part);
+        rc = create_engine(ped, params, devices[g], families, mode, &part);
         if (rc != FS_OK) {
             const std::string keep = g_last_error;
             fs_destroy(front);
@@ -508,20 +558,24 @@ static int create_multi(const fs_pedigree *ped, const fs_params *params, const i
 }
 
 int fs_create_multi(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    return create_multi(ped, params, devices, ndev, false, false, out);
+    return create_multi(ped, params, devices, ndev, false, FamilyMode::NUCLEAR, out);
 }
 
 int fs_create_families(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    return create_multi(ped, params, devices, ndev, true, false, out);
+    return create_multi(ped, params, devices, ndev, true, FamilyMode::NUCLEAR, out);
 }
 
 int fs_create_cohort(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
-    return create_multi(ped, params, devices, ndev, true, true, out);
+    return create_multi(ped, params, devices, ndev, true, FamilyMode::ANY_SHAPE, out);
+}
+
+int fs_create_cohort_bn(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
+    return create_multi(ped, params, devices, ndev, true, FamilyMode::BN, out);
 }
 
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children) {
     if (!e) return fail(FS_E_ARG, "fs_get_families: null engine");
-    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families or fs_create_cohort");
+    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families, fs_create_cohort or fs_create_cohort_bn");
     const FamilyTable &t = e->fam_table;
     if (family) std::memcpy(family, t.family_of.data(), t.family_of.size() * sizeof(int32_t));
     if (n_families) *n_families = t.n_families();
@@ -814,6 +868,11 @@ static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t
         if (rc != FS_OK) return rc;
         B.lut = e->d_pl_table;
     }
+    if (method == FS_METHOD_BN && e->cohort_bn) {
+        FS_CUDA(launch_bn_cohort(e->bn_cohort, B, stream));
+        e->launches += 2 + (int64_t)e->bn_cohort.classes.size();
+        return FS_OK;
+    }
     if (method == FS_METHOD_ES && e->families && e->cohort.n_pf > 0) {
         FS_CUDA(launch_es_cohort(e->cohort, B, stream));
         e->launches += 3;
@@ -1013,7 +1072,8 @@ static int run_host_one(fs_engine *e, int method, int64_t V, const BatchIo &io, 
     cap = std::max<int64_t>(quantum, std::min<int64_t>(cap, 1 << 22)) & ~(quantum - 1);
     cap = std::min<int64_t>(cap, (V + quantum - 1) & ~(quantum - 1));
     // the kernel reads pl / skips single itself
-    const bool fused = method == FS_METHOD_ES && ((e->is_nuclear && !e->force_generic_es) || e->families);
+    const bool fused = (method == FS_METHOD_ES && ((e->is_nuclear && !e->force_generic_es) || e->families)) ||
+                       (method == FS_METHOD_BN && e->cohort_bn);
     const bool want_single = io.single != nullptr || io.single_phred != nullptr;
     int rc = ensure_chunks(e, cap, !io.pl || !fused, io.pl != nullptr, want_single || !fused, io.phred(), io.single_phred != nullptr);
     if (rc != FS_OK) return rc;

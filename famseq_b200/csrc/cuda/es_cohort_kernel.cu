@@ -137,18 +137,32 @@ size_t es_cohort_smem_bytes(int max_vectors, int tb) {
     return (bytes + 15) & ~(size_t)15;
 }
 
-cudaError_t launch_es_cohort(const CohortParams &P, const BatchPtrs &B, cudaStream_t stream) {
-    if (B.V <= 0) return cudaSuccess;
-    switch (P.fam.nc_max) {
-    case 0: launch_head_nc<0>(P.fam, B, stream); break;
-    case 1: launch_head_nc<1>(P.fam, B, stream); break;
-    case 2: launch_head_nc<2>(P.fam, B, stream); break;
-    case 3: launch_head_nc<3>(P.fam, B, stream); break;
-    case 4: launch_head_nc<4>(P.fam, B, stream); break;
-    case 5: launch_head_nc<5>(P.fam, B, stream); break;
+cudaError_t launch_es_cohort_head(const FamiliesParams &P, const BatchPtrs &B, cudaStream_t stream) {
+    switch (P.nc_max) {
+    case 0: launch_head_nc<0>(P, B, stream); break;
+    case 1: launch_head_nc<1>(P, B, stream); break;
+    case 2: launch_head_nc<2>(P, B, stream); break;
+    case 3: launch_head_nc<3>(P, B, stream); break;
+    case 4: launch_head_nc<4>(P, B, stream); break;
+    case 5: launch_head_nc<5>(P, B, stream); break;
     default: return cudaErrorInvalidValue;
     }
-    cudaError_t rc = cudaGetLastError();
+    return cudaGetLastError();
+}
+
+cudaError_t launch_es_cohort_finish(const BatchPtrs &B, int S, cudaStream_t stream) {
+    const int64_t n = B.V * (int64_t)S;
+    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, 148 * 16));
+    if (B.single)
+        es_cohort_finish_kernel<true><<<grid, 256, 0, stream>>>(B, S);
+    else
+        es_cohort_finish_kernel<false><<<grid, 256, 0, stream>>>(B, S);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_es_cohort(const CohortParams &P, const BatchPtrs &B, cudaStream_t stream) {
+    if (B.V <= 0) return cudaSuccess;
+    cudaError_t rc = launch_es_cohort_head(P.fam, B, stream);
     if (rc != cudaSuccess) return rc;
     switch (P.tb) {
     case 128: rc = launch_programs_tb<128>(P, B, stream); break;
@@ -158,13 +172,7 @@ cudaError_t launch_es_cohort(const CohortParams &P, const BatchPtrs &B, cudaStre
     }
     if (rc == cudaSuccess) rc = cudaGetLastError();
     if (rc != cudaSuccess) return rc;
-    const int64_t n = B.V * (int64_t)P.fam.C.s;
-    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, 148 * 16));
-    if (B.single)
-        es_cohort_finish_kernel<true><<<grid, 256, 0, stream>>>(B, P.fam.C.s);
-    else
-        es_cohort_finish_kernel<false><<<grid, 256, 0, stream>>>(B, P.fam.C.s);
-    return cudaGetLastError();
+    return launch_es_cohort_finish(B, P.fam.C.s, stream);
 }
 
 } // namespace famseq

@@ -4,6 +4,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <cuda_runtime.h>
+#include <vector>
 
 #include "../host/bn_plan.hpp"
 #include "../host/es_program.hpp"
@@ -78,6 +79,11 @@ size_t es_cohort_smem_bytes(int max_vectors, int tb);
 // Three launches whatever the number of families: the column pass and nuclear families, the programs, the failure rule.
 // Handles B.pl and B.single == nullptr itself.
 cudaError_t launch_es_cohort(const CohortParams &P, const BatchPtrs &B, cudaStream_t stream);
+// Its first and last launch, for the cohort BN path too: es_cohort_head_kernel (individual-only posteriors, the whole-row
+// gate and failure flag, the nuclear families of P; status := failed | needed << 1) and es_cohort_finish_kernel (NA rows of
+// every failed variant, status := failed).
+cudaError_t launch_es_cohort_head(const FamiliesParams &P, const BatchPtrs &B, cudaStream_t stream);
+cudaError_t launch_es_cohort_finish(const BatchPtrs &B, int S, cudaStream_t stream);
 
 // ---- Bayesian network (bn_kernel.cu) --------------------------------------------------------------
 struct BnParams {
@@ -86,6 +92,28 @@ struct BnParams {
 };
 size_t bn_smem_bytes(const BnParams &P);
 cudaError_t launch_bn(const BnParams &P, const BatchPtrs &B, int sm_count, cudaStream_t stream);
+
+// ---- Bayesian network, cohorts: every family enumerated on its own (bn_cohort_kernel.cu) --------------------------
+// Families of one launch class share the instantiation bn_cohort_kernel<u, independent, factor_leaves> and the block shape
+// (group threads per variant, 256 / group variants per block, 256 threads); they are [begin, end) of the device order.
+struct BnCohortClass {
+    int32_t u, independent, factor_leaves, group;
+    int32_t begin, end;
+    size_t smem; // the largest of bn_cohort_smem_bytes over the class's plans
+};
+struct BnCohortParams {
+    FamiliesParams head;          // n_families = 0: es_cohort_head_kernel's column pass only
+    const BnPlan *plans = nullptr;        // [P] deduplicated plans (device memory, like the arrays below)
+    const int32_t *fam_plan = nullptr;    // [F] plan of each family, device order
+    const int32_t *fam_col_off = nullptr; // [F] offset of its local -> global column map in `cols`
+    const int32_t *cols = nullptr;        // concatenated column maps
+    std::vector<BnCohortClass> classes;   // host side
+};
+// Dynamic shared memory of bn_cohort_kernel for a family of plan `pl`; the staged plan (sizeof(BnPlan)) is static.
+size_t bn_cohort_smem_bytes(const BnPlan &pl);
+// 2 + (launch classes) launches whatever the number of families: the head, one per class, the finish.  Handles B.pl and
+// B.single == nullptr itself.
+cudaError_t launch_bn_cohort(const BnCohortParams &P, const BatchPtrs &B, cudaStream_t stream);
 
 // ---- Gibbs sampler (mcmc_kernel.cu) ---------------------------------------------------------------
 struct McmcParams {

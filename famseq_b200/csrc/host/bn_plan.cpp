@@ -8,12 +8,16 @@
 
 namespace famseq {
 
+std::string bn_too_large_message(int n) {
+    return "The Bayesian-network method enumerates 3^N genotype configurations; N = " + std::to_string(n) +
+           " exceeds the kernel limit of " + std::to_string(BN_MAX_LEVELS) + " members.";
+}
+
 int build_bn_plan(const Pedigree &ped, BnPlan &out, std::string &err) {
     BnPlan p{};
     const int N = ped.n;
     if (N > BN_MAX_LEVELS) {
-        err = "The Bayesian-network method enumerates 3^N genotype configurations; N = " + std::to_string(N) +
-              " exceeds the kernel limit of " + std::to_string(BN_MAX_LEVELS) + " members.";
+        err = bn_too_large_message(N);
         return FS_E_TOO_LARGE;
     }
     p.n_levels = N;

@@ -52,5 +52,7 @@ struct BnPlan {
 
 // Host entry point (bn_plan.cpp): builds the enumeration plan.  Returns FS_OK or FS_E_TOO_LARGE.
 int build_bn_plan(const Pedigree &ped, BnPlan &out, std::string &err);
+// build_bn_plan's refusal of a pedigree of n > BN_MAX_LEVELS members.
+std::string bn_too_large_message(int n);
 
 } // namespace famseq

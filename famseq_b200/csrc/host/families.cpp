@@ -2,9 +2,12 @@
 #include "families.hpp"
 
 #include <algorithm>
+#include <cstring>
 #include <map>
 #include <memory>
 #include <numeric>
+#include <tuple>
+#include <unordered_map>
 
 #include "../../../include/famseq_b200.h"
 #include "es_program.hpp"
@@ -53,9 +56,65 @@ void sub_pedigree(const Pedigree &p, const int *members, int size, std::vector<i
     }
 }
 
+// FamilyMode::BN: every family gets the plan build_bn_plan makes for its own pedigree (the one fs_create builds for the
+// family's rows alone), deduplicated by content; then the device order.
+int build_bn_families(const Pedigree &p, const int32_t *id, const std::vector<int> &start, const std::vector<int> &members,
+                      const std::vector<int> &first_row, FamilyTable &t, std::string &err) {
+    const int F = (int)first_row.size();
+    t.plan.assign(F, -1);
+    t.col_off.assign(F, -1);
+    std::unordered_map<std::string, int32_t> index;
+    std::vector<int> local(p.n, -1);
+    std::vector<int32_t> global_cols;
+    Pedigree sub;
+    BnPlan plan;
+    for (int f = 0; f < F; f++) {
+        const int size = start[f + 1] - start[f];
+        t.n_children[f] = size - (int)std::count_if(members.begin() + start[f], members.begin() + start[f + 1],
+                                                    [&](int i) { return p.founder(i); });
+        std::string why = bn_too_large_message(size);
+        int rc = FS_E_TOO_LARGE;
+        if (size <= BN_MAX_LEVELS) { // no sub-pedigree for a family build_bn_plan refuses by its size
+            sub_pedigree(p, &members[start[f]], size, local, sub, global_cols);
+            rc = build_bn_plan(sub, plan, why);
+        }
+        if (rc != FS_OK) {
+            err = "ped file family of " + std::to_string(id[first_row[f]]) + ": " + why;
+            return rc;
+        }
+        auto hit = index.emplace(std::string(reinterpret_cast<const char *>(&plan), sizeof plan), (int32_t)t.plans.size());
+        if (hit.second) {
+            t.plans.push_back(plan);
+            t.plan_family.push_back(f);
+        }
+        t.plan[f] = hit.first->second;
+        t.col_off[f] = (int32_t)t.cols.size();
+        t.cols.insert(t.cols.end(), global_cols.begin(), global_cols.end());
+    }
+    // device order: by launch class, then by plan, then by first row (a stable sort of the families by (class, plan))
+    auto class_of = [&](int q) {
+        const BnPlan &b = t.plans[q];
+        return std::make_tuple(b.u, b.independent, b.factor_leaves, b.group);
+    };
+    std::vector<int32_t> by_plan(t.plans.size());
+    std::iota(by_plan.begin(), by_plan.end(), 0);
+    std::stable_sort(by_plan.begin(), by_plan.end(), [&](int a, int b) { return class_of(a) < class_of(b); });
+    std::vector<int32_t> rank(t.plans.size());
+    for (size_t k = 0; k < by_plan.size(); k++) rank[by_plan[k]] = (int32_t)k;
+    std::vector<int32_t> at(t.plans.size() + 1, 0);
+    for (int f = 0; f < F; f++) at[rank[t.plan[f]] + 1]++;
+    for (size_t k = 0; k < t.plans.size(); k++) at[k + 1] += at[k];
+    t.bn_order.assign(F, -1);
+    for (int f = 0; f < F; f++) t.bn_order[at[rank[t.plan[f]]]++] = f;
+    for (size_t k = 0; k < by_plan.size(); k++) // at[k] is now the end of the families of plan by_plan[k]
+        if (k + 1 == by_plan.size() || class_of(by_plan[k + 1]) != class_of(by_plan[k])) t.bn_class_end.push_back(at[k]);
+    return FS_OK;
+}
+
 } // namespace
 
-int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err, bool any_shape) {
+int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err, FamilyMode mode) {
+    const bool any_shape = mode == FamilyMode::ANY_SHAPE;
     const int n = p.n;
     // connected families: union-find over the parent links
     std::vector<int> up(n);
@@ -89,9 +148,14 @@ int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::
         std::vector<int> at(start.begin(), start.end() - 1);
         for (int i = 0; i < n; i++) members[at[t.family_of[i]]++] = i;
     }
+    t.n_children.assign(F, 0);
+    if (mode == FamilyMode::BN) {
+        const int rc = build_bn_families(p, id, start, members, first_row, t, err);
+        if (rc == FS_OK) out = std::move(t);
+        return rc;
+    }
     // classify: a lone individual, or two founders (a couple) with 1..5 childless children of both; any other family
     // is refused, or, with any_shape, peeled by a message program of its own
-    t.n_children.assign(F, 0);
     std::vector<int> father(F, -1), mother(F, -1);
     std::vector<char> by_program(F, 0);
     for (int f = 0; f < F; f++) {

@@ -1,12 +1,16 @@
 // families.hpp -- a ped file of many unrelated families (a cohort) split into its connected families for the
 // cohort Elston-Stewart kernels.  Lone individuals and nuclear families (two founders and 1..5 childless children of both)
-// are peeled by cuda/es_families_kernel.cu; with `any_shape`, every other loop-free family of at most 128 members gets an
-// ES message program of its own (host/es_program.cpp), run by cuda/es_cohort_kernel.cu.
+// are peeled by cuda/es_families_kernel.cu; with FamilyMode::ANY_SHAPE, every other loop-free family of at most 128 members
+// gets an ES message program of its own (host/es_program.cpp), run by cuda/es_cohort_kernel.cu.  FamilyMode::BN gives every
+// family, looped ones included, the Bayesian-network plan of its own pedigree (host/bn_plan.cpp), run by
+// cuda/bn_cohort_kernel.cu.
 #pragma once
 
 #include <cstdint>
 #include <string>
 #include <vector>
+
+#include "bn_plan.hpp"
 
 namespace famseq {
 
@@ -37,13 +41,29 @@ struct FamilyTable {
     std::vector<int32_t> pf_order;    // program families sorted by program, then family: the device order
     int32_t max_vectors = 0;          // largest local columns + scratch vectors of any program
 
+    // FamilyMode::BN: every family has a plan (nothing above is filled in but family_of, n_children, col_off and cols).
+    // Plans are deduplicated by content.  Device order: by launch class (u, independent, factor_leaves, group -- one
+    // kernel instantiation and block shape), then by plan, then by first row.
+    std::vector<BnPlan> plans;         // [P]
+    std::vector<int32_t> plan;         // [F] plan of each family
+    std::vector<int32_t> plan_family;  // [P] first family that has the plan (names it in messages)
+    std::vector<int32_t> bn_order;     // [F] the families in device order
+    std::vector<int32_t> bn_class_end; // device-order families [bn_class_end[k-1], bn_class_end[k]) form launch class k
+
     int n_families() const { return (int)n_children.size(); }
     int n_programs() const { return (int)prog_off.size(); }
 };
 
+enum class FamilyMode {
+    NUCLEAR,   // lone individuals and nuclear families only (fs_create_families)
+    ANY_SHAPE, // and an ES message program for every other loop-free family (fs_create_cohort)
+    BN,        // a Bayesian-network plan for every family, loops included (fs_create_cohort_bn)
+};
+
 // FS_OK, or an error with a message naming the first ped id of the first family that is refused: FS_E_TOO_LARGE for a
-// family of another shape (without any_shape) or over a limit of the ES message program, FS_E_LOOP for a looped family
-// (any_shape).  Linear in the number of ped rows plus the compile time of the program families.
-int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err, bool any_shape = false);
+// family of another shape (NUCLEAR), over a limit of the ES message program (ANY_SHAPE) or over BN_MAX_LEVELS members (BN),
+// FS_E_LOOP for a looped family (ANY_SHAPE).  Linear in the number of ped rows plus the compile time of the programs or
+// plans.
+int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::string &err, FamilyMode mode = FamilyMode::NUCLEAR);
 
 } // namespace famseq

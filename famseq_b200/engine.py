@@ -91,6 +91,8 @@ def lib() -> ctypes.CDLL:
         L.fs_get_families.argtypes = [P, P, P, P]
         L.fs_create_cohort.restype = ctypes.c_int
         L.fs_create_cohort.argtypes = [P, P, P, ctypes.c_int, P]
+        L.fs_create_cohort_bn.restype = ctypes.c_int
+        L.fs_create_cohort_bn.argtypes = [P, P, P, ctypes.c_int, P]
         L.fs_get_family_program.restype = ctypes.c_int
         L.fs_get_family_program.argtypes = [P, I32, P, I32, P, P, P, P, P]
         L.fs_run_pl.restype = ctypes.c_int
@@ -137,7 +139,7 @@ EXPORTED_SYMBOLS = ["fs_default_params", "fs_device_count", "fs_create", "fs_des
                     "fs_last_kernel_ms", "fs_bench_fp64_tflops", "fs_get_es_program", "fs_get_gibbs_kernel", "fs_get_es_kernel", "fs_warmup",
                     "fs_create_multi", "fs_run_pl", "fs_run_pl_device", "fs_get_pl_table",
                     "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact",
-                    "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program"]
+                    "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program", "fs_create_cohort_bn"]
 
 
 def _check(rc: int) -> None:
@@ -199,19 +201,21 @@ class Engine:
     every batch call is cut into one contiguous slice of variants per GPU).  families=True takes a cohort ped file of
     nuclear families and lone individuals of any size (fs_create_families, Elston-Stewart only; `device` an int or a
     list, -1 = host side only); cohort=True takes one whose families may also have any other loop-free shape
-    (fs_create_cohort, same rules)."""
+    (fs_create_cohort, same rules).  cohort_bn=True runs the Bayesian network on a cohort ped file of any size, each family
+    (looped ones included, at most 31 members each) enumerated on its own (fs_create_cohort_bn, BN only; `device` as for
+    cohort=True)."""
 
     def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0, families: bool = False,
-                 cohort: bool = False):
+                 cohort: bool = False, cohort_bn: bool = False):
         self._h = ctypes.c_void_p()
         self._keep = [_i32(ids), _i32(mother_ids), _i32(father_ids), _i32(genders), _i32(cols)]
         ped = _Pedigree(len(self._keep[0]), _ptr(self._keep[0]), _ptr(self._keep[1]), _ptr(self._keep[2]),
                         _ptr(self._keep[3]), len(self._keep[4]), _ptr(self._keep[4]))
         self.params = params if params is not None else Params.default()
         self.device = device
-        if families or cohort:
+        if families or cohort or cohort_bn:
             devs = _i32(list(device) if isinstance(device, (list, tuple)) else [device])
-            create = lib().fs_create_cohort if cohort else lib().fs_create_families
+            create = lib().fs_create_cohort_bn if cohort_bn else lib().fs_create_cohort if cohort else lib().fs_create_families
             _check(create(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
         elif isinstance(device, (list, tuple)):
             devs = _i32(list(device))
@@ -250,9 +254,9 @@ class Engine:
         return a, xf, xm, mo, fa
 
     def families(self):
-        """(family[n], n_children[F]) of an engine made with families=True or cohort=True: the family index of each ped row
-        (families numbered by their first row) and each family's number of children (0 = a lone individual; the
-        non-founder members of a family peeled by a message program)."""
+        """(family[n], n_children[F]) of an engine made with families=True, cohort=True or cohort_bn=True: the family index of
+        each ped row (families numbered by their first row) and each family's number of children (0 = a lone individual;
+        the non-founder members of a family peeled by a message program or enumerated by cohort_bn)."""
         nf = ctypes.c_int32(0)
         _check(lib().fs_get_families(self._h, None, ctypes.byref(nf), None))
         fam, kids = np.zeros(self.n, np.int32), np.zeros(nf.value, np.int32)

@@ -120,14 +120,29 @@ int fs_create_families(const fs_pedigree *ped, const fs_params *params, const in
  * validation, error codes, the whole-file LRC gate and failure rule, ES only and the device slicing are those of
  * fs_create_families.  A batch is three kernel launches (one without program families), whatever the number of families. */
 int fs_create_cohort(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
+/* The Bayesian network for cohort ped files: every family -- lone individuals, nuclear and extended families, looped
+ * families too -- is enumerated on its own, with the plan fs_create builds for that family's rows alone (its rows in file
+ * order, its sequenced members as columns in increasing input column); plans are shared by content.  The family split,
+ * ped-row validation, error codes and device slicing are those of fs_create_cohort; no limit on the total member count.
+ * Each member's FPP is its own family's normalised BN marginal: the reference's answer for the whole file, which
+ * factorises by family, up to rounding -- it differs only where the whole-file product of every member's factor leaves
+ * the double range and no single family's product does.  The whole-row rules are those of the cohort ES engines: the LRC
+ * gate uses the pedigree for every sample once one sequenced sample asks for it, and a variant is NA for every sample
+ * (status 1) when an individual-only row sum is <= 0, an unsequenced member's prior fails, or any member of any family
+ * has a BN bin sum <= 0.  Refusals name the family ("ped file family of <first id>: ..."): FS_E_TOO_LARGE for a family
+ * over BN_MAX_LEVELS (31) members or, on a device, one whose plan exceeds shared memory.  BN (-method 1) only: ES and
+ * MCMC runs fail with FS_E_ARG (Elston-Stewart on cohorts is fs_create_cohort).  fs_get_info's bn_levels / bn_group
+ * describe the largest family's plan.  A batch is 2 + (launch classes) kernel launches per chunk, whatever the number of
+ * families: a launch class is the set of plans that share one kernel instantiation and block shape. */
+int fs_create_cohort_bn(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
 /* family[n]: family index of each ped row (families numbered by their first row); n_children[*n_families]: 0 for a lone
- * individual, the number of non-founder members for a family peeled by a program (fs_create_cohort).  Either pointer may
- * be NULL.  FS_E_ARG on an engine that fs_create made. */
+ * individual, the number of non-founder members for a family peeled by a program (fs_create_cohort) or enumerated by
+ * fs_create_cohort_bn.  Either pointer may be NULL.  FS_E_ARG on an engine that fs_create made. */
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children);
 /* Family f of an fs_create_cohort engine (numbered as in fs_get_families): the deduplicated message program it runs
  * (words: capacity in words; *n_words, *n_slots as fs_get_es_program), cols[*n_cols]: the global input column of each of
- * its local columns, *program: the program's index, or -1 for a family the nuclear kernel peels (then *n_words = 0 and
- * *n_cols = 0).  Every pointer may be NULL.  Introspection: tests interpret the programs on the CPU. */
+ * its local columns, *program: the program's index, or -1 for a family the nuclear kernel peels and for every family of an
+ * fs_create_cohort_bn engine (then *n_words = 0 and *n_cols = 0).  Every pointer may be NULL.  Introspection: tests interpret the programs on the CPU. */
 int fs_get_family_program(const fs_engine *e, int32_t f, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
                           int32_t *cols, int32_t *n_cols, int32_t *program);
 

@@ -26,7 +26,7 @@ def gpu_name_and_power():
     return r.stdout.strip().splitlines()[0] if r.returncode == 0 else torch.cuda.get_device_name(0)
 
 
-def time_engine(eng, V, S, compact, steps=20, warmup=3, seed=1):
+def time_engine(eng, V, S, compact, steps=20, warmup=3, seed=1, method=fs.ES):
     """ms per call of run_device / run_pl_device on V variants of S columns (random PLs, device-resident)."""
     g = torch.Generator(device="cuda").manual_seed(seed)
     pl = torch.randint(0, 60, (V, S, 3), device="cuda", dtype=torch.int16, generator=g)
@@ -41,7 +41,7 @@ def time_engine(eng, V, S, compact, steps=20, warmup=3, seed=1):
     stream = torch.cuda.current_stream().cuda_stream
 
     def call():
-        f(fs.ES, V, x.data_ptr(), flags.data_ptr(), post.data_ptr(), single.data_ptr(), gt.data_ptr(), status.data_ptr(), stream=stream)
+        f(method, V, x.data_ptr(), flags.data_ptr(), post.data_ptr(), single.data_ptr(), gt.data_ptr(), status.data_ptr(), stream=stream)
     for _ in range(warmup):
         call()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
