@@ -278,6 +278,7 @@ constexpr size_t kMaxPedigreeMembers = 128; // fs_create's limit
 struct Engine {
     fs_engine *h = nullptr;
     bool family_bn = false; // -familyBN -method 1: fs_create_cohort_bn, for a ped file of any size
+    bool mcmc = false;      // -method 3: fs_create_cohort_mcmc for a ped file past 128 members
     ~Engine() { fs_destroy(h); }
     static std::vector<int> resolve(const std::vector<int> &wanted, int fallback) {
         if (wanted.empty()) return {fallback};
@@ -291,10 +292,13 @@ struct Engine {
             fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
         fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), (int32_t)cm.engine_cols.size(),
                        cm.engine_cols.data()};
-        // ped files past the 128 members of one pedigree: a cohort of loop-free families (ES only)
-        const int rc = family_bn                        ? fs_create_cohort_bn(&fp, &prm, devices.data(), (int)devices.size(), &h)
-                       : id.size() > kMaxPedigreeMembers ? fs_create_cohort(&fp, &prm, devices.data(), (int)devices.size(), &h)
-                                                        : fs_create_multi(&fp, &prm, devices.data(), (int)devices.size(), &h);
+        // ped files past the 128 members of one pedigree: a cohort of families, each on its own chain (MCMC) or a cohort of
+        // loop-free families (ES)
+        const bool cohort = id.size() > kMaxPedigreeMembers;
+        const int rc = family_bn        ? fs_create_cohort_bn(&fp, &prm, devices.data(), (int)devices.size(), &h)
+                       : cohort && mcmc ? fs_create_cohort_mcmc(&fp, &prm, devices.data(), (int)devices.size(), &h)
+                       : cohort         ? fs_create_cohort(&fp, &prm, devices.data(), (int)devices.size(), &h)
+                                        : fs_create_multi(&fp, &prm, devices.data(), (int)devices.size(), &h);
         if (rc != FS_OK) {
             std::cout << fs_last_error() << std::endl;
             g_engine_failed = true;
@@ -745,15 +749,17 @@ bool read_ped(const std::string &path, PedRows &out) {
     return true;
 }
 
-bool check_family(const PedRows &ped, bool family_bn) {
+bool check_family(const PedRows &ped, bool family_bn, bool mcmc) {
     std::vector<int32_t> id(ped.id.begin(), ped.id.end()), mo(ped.mother_id.begin(), ped.mother_id.end()),
         fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
     fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), 0, nullptr};
     fs_engine *h = nullptr;
     const int host_only = -1;
-    const int rc = family_bn                         ? fs_create_cohort_bn(&fp, nullptr, &host_only, 1, &h)
-                   : id.size() > kMaxPedigreeMembers ? fs_create_cohort(&fp, nullptr, &host_only, 1, &h)
-                                                     : fs_create(&fp, nullptr, -1, &h);
+    const bool cohort = id.size() > kMaxPedigreeMembers;
+    const int rc = family_bn        ? fs_create_cohort_bn(&fp, nullptr, &host_only, 1, &h)
+                   : cohort && mcmc ? fs_create_cohort_mcmc(&fp, nullptr, &host_only, 1, &h)
+                   : cohort         ? fs_create_cohort(&fp, nullptr, &host_only, 1, &h)
+                                    : fs_create(&fp, nullptr, -1, &h);
     fs_destroy(h);
     if (rc == FS_OK) return true;
     if (rc == FS_E_GENDER)
@@ -907,6 +913,7 @@ bool run_vcf(const VcfOptions &opt, const PedRows &ped) {
 
     Engine eng;
     eng.family_bn = opt.family_bn && opt.method == 1;
+    eng.mcmc = opt.method == 3;
     EngineStart eng_start(eng, ped, cm, prm, Engine::resolve(opt.devices, opt.device)); // joined before the first engine call (or at the end of an empty input)
     int burn = opt.num_burn_in, rep = opt.num_rep; // file.cpp:644-656
     if (burn < 0) burn = 1000 * real_num_ind;
@@ -1129,6 +1136,7 @@ bool run_lk(const LkOptions &opt, const PedRows &ped) {
 
     Engine eng;
     eng.family_bn = opt.family_bn && opt.method == 1;
+    eng.mcmc = opt.method == 3;
     EngineStart eng_start(eng, ped, cm, prm, Engine::resolve(opt.devices, opt.device)); // joined before the first engine call (or at the end of an empty input)
 
     // decoding and formatting are spread over host threads (see run_vcf / run_pipeline).  The LK driver calls the engine

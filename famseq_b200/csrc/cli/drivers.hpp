@@ -18,8 +18,9 @@ bool read_ped(const std::string &path, PedRows &out);
 
 // Checks the pedigree the way family::init does (half-specified parents, parent genders) before any output
 // is written.  Prints the reference's messages; false = fatal.  family_bn (-familyBN -method 1): the ped file is checked
-// as the cohort Bayesian-network engine takes it (every family on its own, loops allowed).
-bool check_family(const PedRows &ped, bool family_bn);
+// as the cohort Bayesian-network engine takes it (every family on its own, loops allowed); mcmc (-method 3): a ped file past
+// 128 members is checked as the cohort Gibbs sampler takes it (every family on its own, loops allowed).
+bool check_family(const PedRows &ped, bool family_bn, bool mcmc);
 
 bool run_vcf(const VcfOptions &opt, const PedRows &ped);
 bool run_lk(const LkOptions &opt, const PedRows &ped);

@@ -60,8 +60,8 @@ static void help() {
         {"-genoProbK\t", "Genotype probability of three kinds of genotype for autosome in population (Pr(G)) when the variant is in dbSNP. The default value is: 0.45, 0.1 and 0.45."},
         {"-genoProbXN\t", "Genotype probability of two kinds of genotype for chromosome X for male in population (Pr(G)) when the variant is not in dbSNP. The default value is: 0.999 and 0.001."},
         {"-genoProbXK\t", "Genotype probability of two kinds of genotype for chromosome X for male in population (Pr(G)) when the variant is in dbSNP. The default value is: 0.5 and 0.5."},
-        {"-numBurnIn\t", "Number of burn in when the user chooses the MCMC method. The default value is 1,000n, where n is the number of individuals in the pedigree."},
-        {"-numRep\t\t", "Number of iteration times when the user chooses MCMC method. The default value is 20,000n. "},
+        {"-numBurnIn\t", "Number of burn in when the user chooses the MCMC method. The default value is 1,000n, where n is the number of individuals in the pedigree. The default grows with the sample count: for a cohort ped file, give -numBurnIn and -numRep."},
+        {"-numRep\t\t", "Number of iteration times when the user chooses MCMC method. The default value is 20,000n. With -method 3, a ped file of more than 128 individuals runs each family on its own chain, the whole file's chain restricted to that family (families of at most 128 members, loops allowed)."},
         {"-LRC\t\t", "Likelihood ratio criteria (default 1): the pedigree is ignored when every sample's largest normalised likelihood reaches it."},
         {"-l\t\t", "File of tab-separated 'chromosome position' lines; only these positions are processed (vcf mode)."},
         {"-device\t\t", "(this implementation) CUDA device to run on. The default is 0."},
@@ -103,7 +103,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set family." << endl;
             return -1;
         }
-        if (!check_family(ped, opt.family_bn && opt.method == 1)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3)) {
             cout << "Cannot set family." << endl;
             return -1;
         }
@@ -124,7 +124,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set Family." << endl;
             return -1;
         }
-        if (!check_family(ped, opt.family_bn && opt.method == 1)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3)) {
             cout << "Cannot set Family." << endl;
             return -1;
         }

@@ -177,6 +177,9 @@ struct fs_engine {
     // fs_create_cohort_bn: every family enumerated on its own (bn_cohort_kernel.cu), BN only; its device arrays are owned too
     bool cohort_bn = false;
     BnCohortParams bn_cohort;
+    // fs_create_cohort_mcmc: every family's Gibbs chain on its own (mcmc_cohort_kernel.cu), MCMC only; its device arrays are owned too
+    bool cohort_mcmc = false;
+    McmcCohortParams mcmc_cohort;
 };
 
 extern "C" {
@@ -263,17 +266,26 @@ void fs_destroy(fs_engine *e) {
             cudaFree(const_cast<int32_t *>(a));
         cudaFree(const_cast<BnPlan *>(e->bn_cohort.plans));
         for (const int32_t *a : {e->bn_cohort.fam_plan, e->bn_cohort.fam_col_off, e->bn_cohort.cols}) cudaFree(const_cast<int32_t *>(a));
+        cudaFree(const_cast<McmcPlan *>(e->mcmc_cohort.plans));
+        for (const int32_t *a : {e->mcmc_cohort.fam_plan, e->mcmc_cohort.fam_col_off, e->mcmc_cohort.fam_row_off, e->mcmc_cohort.cols,
+                                 e->mcmc_cohort.rows})
+            cudaFree(const_cast<int32_t *>(a));
     }
     delete e;
 }
 
 static const char *creator(bool families, FamilyMode mode) {
     if (!families) return "fs_create";
-    return mode == FamilyMode::BN ? "fs_create_cohort_bn" : mode == FamilyMode::ANY_SHAPE ? "fs_create_cohort" : "fs_create_families";
+    switch (mode) {
+    case FamilyMode::BN: return "fs_create_cohort_bn";
+    case FamilyMode::MCMC: return "fs_create_cohort_mcmc";
+    case FamilyMode::ANY_SHAPE: return "fs_create_cohort";
+    default: return "fs_create_families";
+    }
 }
 
-// fs_create (families == false), and with families == true fs_create_families, fs_create_cohort or fs_create_cohort_bn by
-// `mode`, on one device (-1: host side only).
+// fs_create (families == false), and with families == true fs_create_families, fs_create_cohort, fs_create_cohort_bn or
+// fs_create_cohort_mcmc by `mode`, on one device (-1: host side only).
 static int create_engine(const fs_pedigree *ped, const fs_params *params, int device, bool families, FamilyMode mode, fs_engine **out) {
     const char *who = creator(families, mode);
     if (!ped || !out) return fail(FS_E_ARG, std::string(who) + ": null argument");
@@ -349,6 +361,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
         e->bn_err = e->mcmc_err = "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(t.n_families()) +
                                   " families: only Elston-Stewart (-method 2) runs on ped files over " +
                                   std::to_string(FS_MAX_MEMBERS) + " members";
+        e->mcmc_err += " (the Gibbs sampler on cohorts is fs_create_cohort_mcmc)";
         if (mode == FamilyMode::BN) {
             e->cohort_bn = true;
             e->bn_rc = FS_OK;
@@ -361,6 +374,19 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
             for (int q = 1; q < (int)t.plans.size(); q++)
                 if (t.plans[q].n_levels > t.plans[big].n_levels) big = q;
             if (!t.plans.empty()) e->bn.plan = t.plans[big];
+        }
+        if (mode == FamilyMode::MCMC) {
+            e->cohort_mcmc = true;
+            e->mcmc_rc = FS_OK;
+            e->es_rc = e->bn_rc = FS_E_ARG;
+            e->es_err = e->bn_err = "pedigree of " + std::to_string(e->ped.n) + " members in " + std::to_string(t.n_families()) +
+                                    " families: this engine runs the Gibbs sampler (-method 3) only; Elston-Stewart on cohorts is "
+                                    "fs_create_cohort, the Bayesian network fs_create_cohort_bn";
+            // fs_get_info: the largest family's plan
+            int big = 0;
+            for (int q = 1; q < (int)t.mcmc_plans.size(); q++)
+                if (t.mcmc_plans[q].n > t.mcmc_plans[big].n) big = q;
+            if (!t.mcmc_plans.empty()) e->mcmc.plan = t.mcmc_plans[big];
         }
     }
 
@@ -440,7 +466,7 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
             e->bn_rc = FS_E_TOO_LARGE;
             e->bn_err = "pedigree too large for the BN kernel: per-thread odometer state exceeds shared memory";
         }
-        if (e->mcmc_rc == FS_OK) {
+        if (e->mcmc_rc == FS_OK && !families) {
             e->mcmc_tb = mcmc_pick_block(e->mcmc, e->smem_limit, prop.sharedMemPerMultiprocessor);
             if (e->mcmc_tb == 0) {
                 e->mcmc_rc = FS_E_TOO_LARGE;
@@ -501,13 +527,13 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
                                                         ": pedigree too large for the BN kernel: per-thread odometer state exceeds shared memory");
                     }
                 std::vector<int32_t> fam_plan, fam_col_off;
-                for (int f : t.bn_order) {
+                for (int f : t.plan_order) {
                     fam_plan.push_back(t.plan[f]);
                     fam_col_off.push_back(t.col_off[f]);
                 }
-                for (size_t k = 0, d = 0; k < t.bn_class_end.size(); k++) {
+                for (size_t k = 0, d = 0; k < t.plan_class_end.size(); k++) {
                     const BnPlan &first = t.plans[fam_plan[d]];
-                    BnCohortClass c{first.u, first.independent, first.factor_leaves, first.group, (int32_t)d, t.bn_class_end[k], 0};
+                    BnCohortClass c{first.u, first.independent, first.factor_leaves, first.group, (int32_t)d, t.plan_class_end[k], 0};
                     for (; (int32_t)d < c.end; d++) c.smem = std::max(c.smem, bn_cohort_smem_bytes(t.plans[fam_plan[d]]));
                     P.classes.push_back(c);
                 }
@@ -515,6 +541,36 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
                 if (crc == cudaSuccess) crc = upload(fam_plan, &P.fam_plan);
                 if (crc == cudaSuccess) crc = upload(fam_col_off, &P.fam_col_off);
                 if (crc == cudaSuccess) crc = upload(t.cols, &P.cols);
+            }
+            if (crc == cudaSuccess && e->cohort_mcmc) { // the plans, the column and row maps and the launch classes
+                McmcCohortParams &P = e->mcmc_cohort;
+                P.head = e->fam;
+                std::vector<int32_t> fam_plan, fam_col_off, fam_row_off;
+                for (int f : t.plan_order) {
+                    fam_plan.push_back(t.plan[f]);
+                    fam_col_off.push_back(t.col_off[f]);
+                    fam_row_off.push_back(t.row_off[f]);
+                }
+                for (size_t k = 0, d = 0; k < t.plan_class_end.size(); k++) {
+                    McmcCohortClass c{mcmc_cohort_width(t.mcmc_plans[fam_plan[d]].n), 0, 0, (int32_t)d, t.plan_class_end[k]};
+                    int big = fam_plan[d];
+                    for (; (int32_t)d < c.end; d++)
+                        if (t.mcmc_plans[fam_plan[d]].n > c.n_max) c.n_max = t.mcmc_plans[big = fam_plan[d]].n;
+                    c.tb = mcmc_cohort_pick_block(c.n_max, e->smem_limit, prop.sharedMemPerMultiprocessor);
+                    if (c.tb == 0) {
+                        const int32_t first_id = ped->id[std::find(t.family_of.begin(), t.family_of.end(), t.plan_family[big]) - t.family_of.begin()];
+                        fs_destroy(e);
+                        return fail(FS_E_TOO_LARGE, "ped file family of " + std::to_string(first_id) +
+                                                        ": pedigree too large for the MCMC kernel: chain state exceeds shared memory");
+                    }
+                    P.classes.push_back(c);
+                }
+                crc = upload(t.mcmc_plans, &P.plans);
+                if (crc == cudaSuccess) crc = upload(fam_plan, &P.fam_plan);
+                if (crc == cudaSuccess) crc = upload(fam_col_off, &P.fam_col_off);
+                if (crc == cudaSuccess) crc = upload(fam_row_off, &P.fam_row_off);
+                if (crc == cudaSuccess) crc = upload(t.cols, &P.cols);
+                if (crc == cudaSuccess) crc = upload(t.rows, &P.rows);
             }
             if (crc != cudaSuccess) {
                 fs_destroy(e); // releases what was allocated
@@ -573,9 +629,13 @@ int fs_create_cohort_bn(const fs_pedigree *ped, const fs_params *params, const i
     return create_multi(ped, params, devices, ndev, true, FamilyMode::BN, out);
 }
 
+int fs_create_cohort_mcmc(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out) {
+    return create_multi(ped, params, devices, ndev, true, FamilyMode::MCMC, out);
+}
+
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children) {
     if (!e) return fail(FS_E_ARG, "fs_get_families: null engine");
-    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families, fs_create_cohort or fs_create_cohort_bn");
+    if (!e->families) return fail(FS_E_ARG, "fs_get_families: the engine was not made by fs_create_families or a cohort constructor");
     const FamilyTable &t = e->fam_table;
     if (family) std::memcpy(family, t.family_of.data(), t.family_of.size() * sizeof(int32_t));
     if (n_families) *n_families = t.n_families();
@@ -873,6 +933,11 @@ static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t
         e->launches += 2 + (int64_t)e->bn_cohort.classes.size();
         return FS_OK;
     }
+    if (method == FS_METHOD_MCMC && e->cohort_mcmc) {
+        FS_CUDA(launch_mcmc_cohort(e->mcmc_cohort, B, burn, rep, seed, v_offset, stream));
+        e->launches += 2 + (int64_t)e->mcmc_cohort.classes.size();
+        return FS_OK;
+    }
     if (method == FS_METHOD_ES && e->families && e->cohort.n_pf > 0) {
         FS_CUDA(launch_es_cohort(e->cohort, B, stream));
         e->launches += 3;
@@ -1073,7 +1138,7 @@ static int run_host_one(fs_engine *e, int method, int64_t V, const BatchIo &io, 
     cap = std::min<int64_t>(cap, (V + quantum - 1) & ~(quantum - 1));
     // the kernel reads pl / skips single itself
     const bool fused = (method == FS_METHOD_ES && ((e->is_nuclear && !e->force_generic_es) || e->families)) ||
-                       (method == FS_METHOD_BN && e->cohort_bn);
+                       (method == FS_METHOD_BN && e->cohort_bn) || (method == FS_METHOD_MCMC && e->cohort_mcmc);
     const bool want_single = io.single != nullptr || io.single_phred != nullptr;
     int rc = ensure_chunks(e, cap, !io.pl || !fused, io.pl != nullptr, want_single || !fused, io.phred(), io.single_phred != nullptr);
     if (rc != FS_OK) return rc;

@@ -133,6 +133,34 @@ cudaError_t launch_mcmc(const McmcParams &P, const BatchPtrs &B, int tb, int bur
                         int64_t v_offset, int sm_count, cudaStream_t stream, const McmcTuning &tune, bool fixup = false,
                         unsigned long long *fixup_count = nullptr);
 
+// ---- Gibbs sampler, cohorts: every family's chain on its own (mcmc_cohort_kernel.cu) ----------------------------------
+// Families of one launch class share the genotype-vector width gw (mcmc_cohort_width) and the block size tb; they are
+// [begin, end) of the device order.  n_max, the class's largest family, sizes the shared memory.
+struct McmcCohortClass {
+    int32_t gw, tb, n_max;
+    int32_t begin, end;
+};
+struct McmcCohortParams {
+    FamiliesParams head;                  // n_families = 0: es_cohort_head_kernel's column pass only
+    const McmcPlan *plans = nullptr;      // [P] deduplicated plans (device memory, like the arrays below)
+    const int32_t *fam_plan = nullptr;    // [F] plan of each family, device order
+    const int32_t *fam_col_off = nullptr; // [F] offset of its local -> global column map in `cols`
+    const int32_t *fam_row_off = nullptr; // [F] offset of its local member -> global ped row map in `rows`
+    const int32_t *cols = nullptr;        // concatenated column maps
+    const int32_t *rows = nullptr;        // concatenated row maps
+    std::vector<McmcCohortClass> classes; // host side
+};
+// Dynamic shared memory of mcmc_cohort_kernel for families of at most n members at block size tb (the staged plan and row /
+// column maps, MCMC_COHORT_STATIC_SMEM bytes, are static).
+size_t mcmc_cohort_smem_bytes(int n, int tb);
+// mcmc_pick_block's rule for the cohort kernel: the block size that keeps the most chains resident per SM for families of
+// at most n members; 0 when not even 32 chains fit.
+int mcmc_cohort_pick_block(int n, size_t smem_limit, size_t smem_per_sm);
+// 2 + (launch classes) launches whatever the number of families: the head, one per class, the finish.  Handles B.pl and
+// B.single == nullptr itself.
+cudaError_t launch_mcmc_cohort(const McmcCohortParams &P, const BatchPtrs &B, int burn, int rep, uint64_t seed, int64_t v_offset,
+                               cudaStream_t stream);
+
 // ---- compact input (engine.cu) ----------------------------------------------------------------------
 // lk[k] = lut[pl[k]] for k < n: expands fs_run_pl input for the kernels that read FP64 likelihoods.
 cudaError_t launch_pl_decode(const uint16_t *pl, const double *lut, double *lk, int64_t n, cudaStream_t stream);

@@ -31,72 +31,12 @@
 //   * persistent blocks loop over tiles of TB variants.
 #include <algorithm>
 
-#include "common.cuh"
 #include "kernels.hpp"
+#include "mcmc_step.cuh"
 
 namespace famseq {
 
 namespace {
-
-constexpr int kCopies = 16;      // replicas of every table entry
-constexpr int kEntries = 81 + 27; // 3 x 27 transmission entries followed by 27 ones
-constexpr int kOnes = 81;
-
-__device__ __forceinline__ double lds64(uint32_t shared_addr) {
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(shared_addr));
-    return v;
-}
-
-__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
-                                              uint32_t &o0, uint32_t &o1, uint32_t &o2, uint32_t &o3) {
-#pragma unroll
-    for (int r = 0; r < 10; r++) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-        c0 = n0;
-        c1 = lo1;
-        c2 = n2;
-        c3 = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-    o0 = c0;
-    o1 = c1;
-    o2 = c2;
-    o3 = c3;
-}
-
-// genotype vector, 2 bits per member in GW 64-bit words (GW = 2: up to 64 members, GW = 4: up to 128); the member index
-// is warp-uniform
-template <int GW> struct Genotypes {
-    uint64_t w[GW];
-    __device__ __forceinline__ uint64_t word(int i) const {
-        if (GW == 2) return i < 32 ? w[0] : w[1];
-        return i < 64 ? (i < 32 ? w[0] : w[1]) : (i < 96 ? w[2] : w[GW - 1]);
-    }
-    __device__ __forceinline__ int get(int i) const { return (int)((word(i) >> (2 * (i & 31))) & 3u); }
-    __device__ __forceinline__ void set(int i, int g) {
-        const uint64_t m = 3ull << (2 * (i & 31)), v = (uint64_t)g << (2 * (i & 31));
-#pragma unroll
-        for (int k = 0; k < GW; k++)
-            if ((i >> 5) == k) w[k] = (w[k] & ~m) | v;
-    }
-};
-
-// 1/s to ~1 ulp: hardware seed (MUFU.RCP64H) + two Newton steps; outside the safe range the IEEE divide.
-__device__ __forceinline__ double fast_reciprocal(double s) {
-    double x;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(s));
-    double e = fma(-s, x, 1.0);
-    x = fma(x, e, x);
-    e = fma(-s, x, 1.0);
-    x = fma(x, e, x);
-    // rare: not a positive normal number with exponent in [-963, 963) (integer-pipe test on the high word)
-    if (!(((unsigned)__double2hiint(s) - 0x03c00000u) < 0x78600000u)) x = 1.0 / s;
-    return x;
-}
 
 // WGLOBAL = false: own factors in shared memory (small pedigrees: every chain of a full SM fits).
 // WGLOBAL = true : own factors in the global scratch next to the accumulators, read one member ahead through L2;
@@ -182,12 +122,9 @@ __global__ void __launch_bounds__(TB) mcmc_kernel(const __grid_constant__ McmcPa
         for (int i = 0; i < N; i++) {
             const uint32_t d = pl.member[i];
             const int col = pl.col[i];
-            const bool founder = (d >> 14) & 1u, male = (d >> 15) & 1u;
 #pragma unroll
             for (int g = 0; g < 3; g++) {
-                const double lk = col >= 0 ? lkv[col * 3 + g] : 1.0;
-                const double base = founder ? 1000000.0 * (male ? pick3(pr.m, g) : pick3(pr.a, g)) : 1000000.0;
-                w[(i * 3 + g) * TB] = base * lk;
+                w[(i * 3 + g) * TB] = gibbs_own_factor(d, pr, g, col >= 0 ? lkv[col * 3 + g] : 1.0);
                 acc[(size_t)((i * 3 + g) * TB)] = 0.0;
             }
         }
@@ -204,9 +141,7 @@ __global__ void __launch_bounds__(TB) mcmc_kernel(const __grid_constant__ McmcPa
             cur.set(i, (int)(u % 3u));
         }
 
-        // ---- sweeps ---------------------------------------------------------------------------------------------
-        // The step is written branch-light: founders and missing children multiply by a row of ones, the first two
-        // children are handled in line, shared memory is addressed with 32-bit shared-window addresses.
+        // ---- sweeps (the step: mcmc_step.cuh) ---------------------------------------------------------------------
         asm volatile("" ::: "memory");
         double nw0 = 0.0, nw1 = 0.0, nw2 = 0.0; // WGLOBAL: own factors of the next member, fetched one step ahead
         if constexpr (WGLOBAL) {
@@ -219,7 +154,6 @@ __global__ void __launch_bounds__(TB) mcmc_kernel(const __grid_constant__ McmcPa
             const bool sampling = sweep > burn;
             for (int i = 0; i < N; i++) {
                 const uint32_t d = pl.member[i];
-                const bool male = (d >> 15) & 1u, founder = (d >> 14) & 1u;
                 double w0, w1, w2;
                 if constexpr (WGLOBAL) {
                     w0 = nw0;
@@ -235,55 +169,15 @@ __global__ void __launch_bounds__(TB) mcmc_kernel(const __grid_constant__ McmcPa
                     w1 = lds64(wa + TB * 8);
                     w2 = lds64(wa + 2 * TB * 8);
                 }
-                const int xkind = male ? 2 * 27 : 27; // chrX table of this member / of a child, by sex
-                {   // own factor: transmission from the parents' current genotypes (a row of ones for founders)
-                    const int row = cur.get(d & 127u) * 3 + cur.get((d >> 7) & 127u);
-                    const int e = founder ? kOnes : (chrx ? xkind : 0) + row;
-                    const uint32_t ta = tab_addr + (uint32_t)e * (kCopies * 8u);
-                    w0 *= lds64(ta);
-                    w1 *= lds64(ta + 9 * kCopies * 8);
-                    w2 *= lds64(ta + 18 * kCopies * 8);
-                }
-                const int lb = (d >> 16) & 0xffu;
-                const int n_links = (!chrx || male) ? (int)(d >> 24) : 0; // chrX: only males get the children factor
-                const uint32_t step = male ? kCopies * 8u : 3u * kCopies * 8u;     // this member sits in the father slot when male
-                auto child_entry = [&](int k) -> int {
-                    const uint32_t l = pl.link[k];
-                    const int kind = chrx ? (((l >> 14) & 1u) ? 2 * 27 : 27) : 0;
-                    const int other = cur.get((l >> 7) & 127u);
-                    return kind + cur.get(l & 127u) * 9 + (male ? other * 3 : other);
-                };
-                {   // first two children in line (a row of ones when there are fewer)
-                    const int e0 = n_links > 0 ? child_entry(lb) : kOnes;
-                    const int e1 = n_links > 1 ? child_entry(lb + 1) : kOnes;
-                    const uint32_t a0 = tab_addr + (uint32_t)e0 * (kCopies * 8u), a1 = tab_addr + (uint32_t)e1 * (kCopies * 8u);
-                    const double x0 = lds64(a0), x1 = lds64(a0 + step), x2 = lds64(a0 + 2 * step);
-                    const double y0 = lds64(a1), y1 = lds64(a1 + step), y2 = lds64(a1 + 2 * step);
-                    w0 = (w0 * x0) * y0;
-                    w1 = (w1 * x1) * y1;
-                    w2 = (w2 * x2) * y2;
-                }
-                for (int k = lb + 2; k < lb + n_links; k++) { // third and later children
-                    const uint32_t a0 = tab_addr + (uint32_t)child_entry(k) * (kCopies * 8u);
-                    w0 *= lds64(a0);
-                    w1 *= lds64(a0 + step);
-                    w2 *= lds64(a0 + 2 * step);
-                }
-                const double sum = (w0 + w1) + w2;
+                const double sum = gibbs_weights(d, pl.link, cur, chrx, tab_addr, w0, w1, w2);
                 if ((i & 3) == 0) philox4x32_10((uint32_t)sweep, (uint32_t)(i >> 2), gv_lo, gv_hi, k0, k1, r0, r1, r2, r3);
                 const uint32_t u = r0; // words are consumed in order: rotate the block
                 r0 = r1;
                 r1 = r2;
                 r2 = r3;
-                const double rd = ((double)(u >> 1) + 0.5) * (1.0 / 2147483648.0); // 31 bits, like the reference's rand() / RAND_MAX
-                // rd < w0/sum and rd > 1 - w2/sum decided without the division; a non-positive sum means all-zero
-                // weights in the reference, which then draws genotype 1 (family.cpp:2142-2173)
-                const double thr = rd * sum;
-                int g = (thr < w0) ? 0 : ((thr > sum - w2) ? 2 : 1);
-                if (!(sum > 0.0)) g = 1;
-                cur.set(i, g);
-                if (sampling) { // family.cpp:2175-2178, Rao-Blackwellised; all-zero weights add nothing
-                    const double inv = sum > 0.0 ? fast_reciprocal(sum) : 0.0;
+                cur.set(i, gibbs_draw(u, sum, w0, w2));
+                if (sampling) { // family.cpp:2175-2178, Rao-Blackwellised
+                    const double inv = gibbs_inv(sum);
                     double *a = acc + (size_t)((i * 3) * TB);
                     atomicAdd(a, w0 * inv);
                     atomicAdd(a + TB, w1 * inv);

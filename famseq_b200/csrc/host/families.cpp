@@ -56,10 +56,13 @@ void sub_pedigree(const Pedigree &p, const int *members, int size, std::vector<i
     }
 }
 
-// FamilyMode::BN: every family gets the plan build_bn_plan makes for its own pedigree (the one fs_create builds for the
-// family's rows alone), deduplicated by content; then the device order.
-int build_bn_families(const Pedigree &p, const int32_t *id, const std::vector<int> &start, const std::vector<int> &members,
-                      const std::vector<int> &first_row, FamilyTable &t, std::string &err) {
+// FamilyMode::BN and MCMC: every family gets the plan `build(sub, size, plan, why)` makes for its own pedigree (the one
+// fs_create builds for the family's rows alone), deduplicated by content; then the device order by launch class
+// (`class_of(plan)`), plan and first row.
+template <class Plan, class Build, class ClassOf>
+int build_plan_families(const Pedigree &p, const int32_t *id, const std::vector<int> &start, const std::vector<int> &members,
+                        const std::vector<int> &first_row, FamilyTable &t, std::vector<Plan> &plans, Build build, ClassOf class_of,
+                        std::string &err) {
     const int F = (int)first_row.size();
     t.plan.assign(F, -1);
     t.col_off.assign(F, -1);
@@ -67,24 +70,20 @@ int build_bn_families(const Pedigree &p, const int32_t *id, const std::vector<in
     std::vector<int> local(p.n, -1);
     std::vector<int32_t> global_cols;
     Pedigree sub;
-    BnPlan plan;
+    Plan plan;
     for (int f = 0; f < F; f++) {
         const int size = start[f + 1] - start[f];
         t.n_children[f] = size - (int)std::count_if(members.begin() + start[f], members.begin() + start[f + 1],
                                                     [&](int i) { return p.founder(i); });
-        std::string why = bn_too_large_message(size);
-        int rc = FS_E_TOO_LARGE;
-        if (size <= BN_MAX_LEVELS) { // no sub-pedigree for a family build_bn_plan refuses by its size
-            sub_pedigree(p, &members[start[f]], size, local, sub, global_cols);
-            rc = build_bn_plan(sub, plan, why);
-        }
+        std::string why;
+        const int rc = build(&members[start[f]], size, local, sub, global_cols, plan, why);
         if (rc != FS_OK) {
             err = "ped file family of " + std::to_string(id[first_row[f]]) + ": " + why;
             return rc;
         }
-        auto hit = index.emplace(std::string(reinterpret_cast<const char *>(&plan), sizeof plan), (int32_t)t.plans.size());
+        auto hit = index.emplace(std::string(reinterpret_cast<const char *>(&plan), sizeof plan), (int32_t)plans.size());
         if (hit.second) {
-            t.plans.push_back(plan);
+            plans.push_back(plan);
             t.plan_family.push_back(f);
         }
         t.plan[f] = hit.first->second;
@@ -92,22 +91,19 @@ int build_bn_families(const Pedigree &p, const int32_t *id, const std::vector<in
         t.cols.insert(t.cols.end(), global_cols.begin(), global_cols.end());
     }
     // device order: by launch class, then by plan, then by first row (a stable sort of the families by (class, plan))
-    auto class_of = [&](int q) {
-        const BnPlan &b = t.plans[q];
-        return std::make_tuple(b.u, b.independent, b.factor_leaves, b.group);
-    };
-    std::vector<int32_t> by_plan(t.plans.size());
+    std::vector<int32_t> by_plan(plans.size());
     std::iota(by_plan.begin(), by_plan.end(), 0);
-    std::stable_sort(by_plan.begin(), by_plan.end(), [&](int a, int b) { return class_of(a) < class_of(b); });
-    std::vector<int32_t> rank(t.plans.size());
+    std::stable_sort(by_plan.begin(), by_plan.end(), [&](int a, int b) { return class_of(plans[a]) < class_of(plans[b]); });
+    std::vector<int32_t> rank(plans.size());
     for (size_t k = 0; k < by_plan.size(); k++) rank[by_plan[k]] = (int32_t)k;
-    std::vector<int32_t> at(t.plans.size() + 1, 0);
+    std::vector<int32_t> at(plans.size() + 1, 0);
     for (int f = 0; f < F; f++) at[rank[t.plan[f]] + 1]++;
-    for (size_t k = 0; k < t.plans.size(); k++) at[k + 1] += at[k];
-    t.bn_order.assign(F, -1);
-    for (int f = 0; f < F; f++) t.bn_order[at[rank[t.plan[f]]]++] = f;
+    for (size_t k = 0; k < plans.size(); k++) at[k + 1] += at[k];
+    t.plan_order.assign(F, -1);
+    for (int f = 0; f < F; f++) t.plan_order[at[rank[t.plan[f]]]++] = f;
     for (size_t k = 0; k < by_plan.size(); k++) // at[k] is now the end of the families of plan by_plan[k]
-        if (k + 1 == by_plan.size() || class_of(by_plan[k + 1]) != class_of(by_plan[k])) t.bn_class_end.push_back(at[k]);
+        if (k + 1 == by_plan.size() || class_of(plans[by_plan[k + 1]]) != class_of(plans[by_plan[k]]))
+            t.plan_class_end.push_back(at[k]);
     return FS_OK;
 }
 
@@ -150,9 +146,38 @@ int build_families(const Pedigree &p, const int32_t *id, FamilyTable &out, std::
     }
     t.n_children.assign(F, 0);
     if (mode == FamilyMode::BN) {
-        const int rc = build_bn_families(p, id, start, members, first_row, t, err);
+        auto build = [&](const int *rows, int size, std::vector<int> &local, Pedigree &sub, std::vector<int32_t> &global_cols,
+                         BnPlan &plan, std::string &why) {
+            if (size > BN_MAX_LEVELS) { // no sub-pedigree for a family build_bn_plan refuses by its size
+                why = bn_too_large_message(size);
+                return (int)FS_E_TOO_LARGE;
+            }
+            sub_pedigree(p, rows, size, local, sub, global_cols);
+            return build_bn_plan(sub, plan, why);
+        };
+        auto class_of = [](const BnPlan &b) { return std::make_tuple(b.u, b.independent, b.factor_leaves, b.group); };
+        const int rc = build_plan_families(p, id, start, members, first_row, t, t.plans, build, class_of, err);
         if (rc == FS_OK) out = std::move(t);
         return rc;
+    }
+    if (mode == FamilyMode::MCMC) {
+        auto build = [&](const int *rows, int size, std::vector<int> &local, Pedigree &sub, std::vector<int32_t> &global_cols,
+                         McmcPlan &plan, std::string &why) {
+            if (size > MCMC_MAX_MEMBERS) {
+                why = std::to_string(size) + " members; the MCMC kernel supports families of up to " + std::to_string(MCMC_MAX_MEMBERS) +
+                      " members";
+                return (int)FS_E_TOO_LARGE;
+            }
+            sub_pedigree(p, rows, size, local, sub, global_cols);
+            return build_mcmc_plan(sub, plan, why);
+        };
+        auto class_of = [](const McmcPlan &m) { return mcmc_cohort_width(m.n); };
+        const int rc = build_plan_families(p, id, start, members, first_row, t, t.mcmc_plans, build, class_of, err);
+        if (rc != FS_OK) return rc;
+        t.rows.assign(members.begin(), members.end());
+        t.row_off.assign(start.begin(), start.end());
+        out = std::move(t);
+        return FS_OK;
     }
     // classify: a lone individual, or two founders (a couple) with 1..5 childless children of both; any other family
     // is refused, or, with any_shape, peeled by a message program of its own

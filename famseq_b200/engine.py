@@ -93,6 +93,8 @@ def lib() -> ctypes.CDLL:
         L.fs_create_cohort.argtypes = [P, P, P, ctypes.c_int, P]
         L.fs_create_cohort_bn.restype = ctypes.c_int
         L.fs_create_cohort_bn.argtypes = [P, P, P, ctypes.c_int, P]
+        L.fs_create_cohort_mcmc.restype = ctypes.c_int
+        L.fs_create_cohort_mcmc.argtypes = [P, P, P, ctypes.c_int, P]
         L.fs_get_family_program.restype = ctypes.c_int
         L.fs_get_family_program.argtypes = [P, I32, P, I32, P, P, P, P, P]
         L.fs_run_pl.restype = ctypes.c_int
@@ -139,7 +141,8 @@ EXPORTED_SYMBOLS = ["fs_default_params", "fs_device_count", "fs_create", "fs_des
                     "fs_last_kernel_ms", "fs_bench_fp64_tflops", "fs_get_es_program", "fs_get_gibbs_kernel", "fs_get_es_kernel", "fs_warmup",
                     "fs_create_multi", "fs_run_pl", "fs_run_pl_device", "fs_get_pl_table",
                     "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact",
-                    "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program", "fs_create_cohort_bn"]
+                    "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program", "fs_create_cohort_bn",
+                    "fs_create_cohort_mcmc"]
 
 
 def _check(rc: int) -> None:
@@ -203,19 +206,22 @@ class Engine:
     list, -1 = host side only); cohort=True takes one whose families may also have any other loop-free shape
     (fs_create_cohort, same rules).  cohort_bn=True runs the Bayesian network on a cohort ped file of any size, each family
     (looped ones included, at most 31 members each) enumerated on its own (fs_create_cohort_bn, BN only; `device` as for
-    cohort=True)."""
+    cohort=True).  cohort_mcmc=True runs the Gibbs sampler on a cohort ped file of any size, each family (looped ones
+    included, at most 128 members each) on its own chain, which is the whole file's chain restricted to that family
+    (fs_create_cohort_mcmc, MCMC only; `device` as for cohort=True)."""
 
     def __init__(self, ids, mother_ids, father_ids, genders, cols, params: Params | None = None, device=0, families: bool = False,
-                 cohort: bool = False, cohort_bn: bool = False):
+                 cohort: bool = False, cohort_bn: bool = False, cohort_mcmc: bool = False):
         self._h = ctypes.c_void_p()
         self._keep = [_i32(ids), _i32(mother_ids), _i32(father_ids), _i32(genders), _i32(cols)]
         ped = _Pedigree(len(self._keep[0]), _ptr(self._keep[0]), _ptr(self._keep[1]), _ptr(self._keep[2]),
                         _ptr(self._keep[3]), len(self._keep[4]), _ptr(self._keep[4]))
         self.params = params if params is not None else Params.default()
         self.device = device
-        if families or cohort or cohort_bn:
+        if families or cohort or cohort_bn or cohort_mcmc:
             devs = _i32(list(device) if isinstance(device, (list, tuple)) else [device])
-            create = lib().fs_create_cohort_bn if cohort_bn else lib().fs_create_cohort if cohort else lib().fs_create_families
+            create = (lib().fs_create_cohort_mcmc if cohort_mcmc else lib().fs_create_cohort_bn if cohort_bn
+                      else lib().fs_create_cohort if cohort else lib().fs_create_families)
             _check(create(ctypes.byref(ped), ctypes.byref(self.params), _ptr(devs), len(devs), ctypes.byref(self._h)))
         elif isinstance(device, (list, tuple)):
             devs = _i32(list(device))
@@ -254,9 +260,9 @@ class Engine:
         return a, xf, xm, mo, fa
 
     def families(self):
-        """(family[n], n_children[F]) of an engine made with families=True, cohort=True or cohort_bn=True: the family index of
+        """(family[n], n_children[F]) of an engine made with families=True or a cohort constructor: the family index of
         each ped row (families numbered by their first row) and each family's number of children (0 = a lone individual;
-        the non-founder members of a family peeled by a message program or enumerated by cohort_bn)."""
+        the non-founder members of a family peeled by a message program or run by cohort_bn / cohort_mcmc)."""
         nf = ctypes.c_int32(0)
         _check(lib().fs_get_families(self._h, None, ctypes.byref(nf), None))
         fam, kids = np.zeros(self.n, np.int32), np.zeros(nf.value, np.int32)

@@ -135,14 +135,33 @@ int fs_create_cohort(const fs_pedigree *ped, const fs_params *params, const int 
  * describe the largest family's plan.  A batch is 2 + (launch classes) kernel launches per chunk, whatever the number of
  * families: a launch class is the set of plans that share one kernel instantiation and block shape. */
 int fs_create_cohort_bn(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
+/* The Gibbs sampler (MCMC) for cohort ped files: every family -- lone individuals, nuclear and extended families, looped
+ * families too -- runs its own chain, with the plan fs_create builds for that family's rows alone; plans are shared by
+ * content.  The family split, ped-row validation, error codes and device slicing are those of fs_create_cohort_bn; no limit
+ * on the total member count.  The chains are those of the whole file: fs_create's sampler visits the members in ped
+ * order, a member's full conditional reads only its own family, and a member's random word depends only on (seed, global
+ * site, sweep, global ped row).  So each family's chain, with its members swept in increasing ped row and its words drawn
+ * with their global ped rows, is the whole-file chain restricted to that family, and the outputs are byte-identical to
+ * fs_create's table-driven sampler (FAMSEQ_MCMC_JIT=0) on any file fs_create takes.  The whole-row rules are those of the
+ * cohort ES engines: the LRC gate uses the pedigree for every sample once one sequenced sample asks for it, and a variant
+ * is NA for every sample (status 1) when an individual-only row sum is <= 0, an unsequenced member's prior fails, or any
+ * member of any family ends with a posterior row summing to <= 0.  Families with no sequenced member run their chains
+ * too.  Refusals name the family ("ped file family of <first id>: ..."): FS_E_TOO_LARGE for a family over
+ * MCMC_MAX_MEMBERS (128) members or, on a device, one whose chain state exceeds shared memory.  MCMC (-method 3) only:
+ * ES and BN runs fail with FS_E_ARG (fs_create_cohort, fs_create_cohort_bn).  fs_get_info's mcmc_links describes the
+ * largest family's plan, and gibbs_generator stays 0 (no generated kernel).  A batch is 2 + (launch classes) kernel
+ * launches per chunk, whatever the number of families: a launch class is the set of families of one genotype-vector
+ * width (at most 32, 64 or 128 members). */
+int fs_create_cohort_mcmc(const fs_pedigree *ped, const fs_params *params, const int *devices, int ndev, fs_engine **out);
 /* family[n]: family index of each ped row (families numbered by their first row); n_children[*n_families]: 0 for a lone
  * individual, the number of non-founder members for a family peeled by a program (fs_create_cohort) or enumerated by
- * fs_create_cohort_bn.  Either pointer may be NULL.  FS_E_ARG on an engine that fs_create made. */
+ * fs_create_cohort_bn or run by fs_create_cohort_mcmc.  Either pointer may be NULL.  FS_E_ARG on an engine that fs_create
+ * made. */
 int fs_get_families(const fs_engine *e, int32_t *family, int32_t *n_families, int32_t *n_children);
 /* Family f of an fs_create_cohort engine (numbered as in fs_get_families): the deduplicated message program it runs
  * (words: capacity in words; *n_words, *n_slots as fs_get_es_program), cols[*n_cols]: the global input column of each of
  * its local columns, *program: the program's index, or -1 for a family the nuclear kernel peels and for every family of an
- * fs_create_cohort_bn engine (then *n_words = 0 and *n_cols = 0).  Every pointer may be NULL.  Introspection: tests interpret the programs on the CPU. */
+ * fs_create_cohort_bn or fs_create_cohort_mcmc engine (then *n_words = 0 and *n_cols = 0).  Every pointer may be NULL.  Introspection: tests interpret the programs on the CPU. */
 int fs_get_family_program(const fs_engine *e, int32_t f, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
                           int32_t *cols, int32_t *n_cols, int32_t *program);
 
