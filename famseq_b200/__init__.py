@@ -5,5 +5,5 @@ built from famseq_b200/csrc for sm_100a.  This package only binds the library fo
 and generates synthetic inputs; it contains no CPU implementation of the engine.
 """
 from . import synth  # noqa: F401
-from .engine import (BN, ES, MCMC, FLAG_CHRX, FLAG_KNOWN, Engine, FamSeqError, Params, PhredResult, Result,  # noqa: F401
+from .engine import (BN, BN_PEEL, ES, MCMC, FLAG_CHRX, FLAG_KNOWN, Engine, FamSeqError, Params, PhredResult, Result,  # noqa: F401
                      device_count, lib, phred_text, phred_text_exact)

@@ -749,7 +749,19 @@ bool read_ped(const std::string &path, PedRows &out) {
     return true;
 }
 
-bool check_family(const PedRows &ped, bool family_bn, bool mcmc) {
+int engine_method(const CommonOptions &opt) { return opt.peel_loops && opt.method == 1 ? FS_METHOD_BN_PEEL : opt.method; }
+
+bool check_family(const PedRows &ped, bool family_bn, bool mcmc, bool peel) {
+    if (peel && family_bn) {
+        std::cout << "-peelLoops and -familyBN cannot be used together: -peelLoops computes the Bayesian network of the whole "
+                     "ped file (at most " << kMaxPedigreeMembers << " individuals) by conditioned peeling." << std::endl;
+        return false;
+    }
+    if (peel && ped.id.size() > kMaxPedigreeMembers) {
+        std::cout << "-peelLoops takes ped files of at most " << kMaxPedigreeMembers << " individuals; this one has "
+                  << ped.id.size() << ". Use -familyBN for ped files of many families." << std::endl;
+        return false;
+    }
     std::vector<int32_t> id(ped.id.begin(), ped.id.end()), mo(ped.mother_id.begin(), ped.mother_id.end()),
         fa(ped.father_id.begin(), ped.father_id.end()), ge(ped.gender.begin(), ped.gender.end());
     fs_pedigree fp{(int32_t)id.size(), id.data(), mo.data(), fa.data(), ge.data(), 0, nullptr};
@@ -760,7 +772,14 @@ bool check_family(const PedRows &ped, bool family_bn, bool mcmc) {
                    : cohort && mcmc ? fs_create_cohort_mcmc(&fp, nullptr, &host_only, 1, &h)
                    : cohort         ? fs_create_cohort(&fp, nullptr, &host_only, 1, &h)
                                     : fs_create(&fp, nullptr, -1, &h);
+    // the conditioned program is refused (too many loop breakers, too long) at run time, so ask for it here
+    const int prc = rc == FS_OK && peel ? fs_get_bn_peel_program(h, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr) : rc;
     fs_destroy(h);
+    if (prc != FS_OK && rc == FS_OK) {
+        std::cout << fs_last_error() << std::endl;
+        std::cout << "Cannot initiate family. Please check ped file." << std::endl;
+        return false;
+    }
     if (rc == FS_OK) return true;
     if (rc == FS_E_GENDER)
         std::cerr << fs_last_error() << std::endl; // family.cpp:208,213 write to cerr
@@ -1068,7 +1087,7 @@ bool run_vcf(const VcfOptions &opt, const PedRows &ped) {
     Lines in(data);
     // the reference stops at the first line shorter than two characters; header lines are not records
     auto accept = [](sv line) { return line.size() < 2 ? 0 : (line[0] == '#' ? 2 : 1); };
-    const PipelineSetup setup{&eng, &eng_start, S, opt.method, burn, rep, opt.seed, &writer};
+    const PipelineSetup setup{&eng, &eng_start, S, engine_method(opt), burn, rep, opt.seed, &writer};
     bool ok = run_pipeline(in, setup, accept, parse_range, format_range);
     {
         const double t0 = now();
@@ -1214,7 +1233,7 @@ bool run_lk(const LkOptions &opt, const PedRows &ped) {
     writer.push(std::move(out)); // header
     out.clear();
     auto accept = [](sv line) { return line.size() < 2 ? 0 : 1; };
-    const PipelineSetup setup{&eng, &eng_start, S, opt.method, opt.num_burn_in, opt.num_rep, opt.seed, &writer};
+    const PipelineSetup setup{&eng, &eng_start, S, engine_method(opt), opt.num_burn_in, opt.num_rep, opt.seed, &writer};
     bool ok = run_pipeline(in, setup, accept, parse_range, format_range);
     {
         const double t0 = now();

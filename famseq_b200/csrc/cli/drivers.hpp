@@ -20,7 +20,11 @@ bool read_ped(const std::string &path, PedRows &out);
 // is written.  Prints the reference's messages; false = fatal.  family_bn (-familyBN -method 1): the ped file is checked
 // as the cohort Bayesian-network engine takes it (every family on its own, loops allowed); mcmc (-method 3): a ped file past
 // 128 members is checked as the cohort Gibbs sampler takes it (every family on its own, loops allowed).
-bool check_family(const PedRows &ped, bool family_bn, bool mcmc);
+// peel (-peelLoops -method 1): the pedigree must be one fs_create takes (at most 128 members, not with -familyBN) and its
+// conditioned program must not be refused.
+bool check_family(const PedRows &ped, bool family_bn, bool mcmc, bool peel);
+// The engine method of the options: FS_METHOD_BN_PEEL for -method 1 -peelLoops, the -method value otherwise.
+int engine_method(const CommonOptions &opt);
 
 bool run_vcf(const VcfOptions &opt, const PedRows &ped);
 bool run_lk(const LkOptions &opt, const PedRows &ped);

@@ -66,6 +66,7 @@ static void help() {
         {"-l\t\t", "File of tab-separated 'chromosome position' lines; only these positions are processed (vcf mode)."},
         {"-device\t\t", "(this implementation) CUDA device to run on. The default is 0."},
         {"-seed\t\t", "(this implementation) Seed of the counter-based random number generator of the MCMC method. The default is 1."},
+        {"-peelLoops\t", "(this implementation) With -method 1: compute the Bayesian network's exact posteriors by Elston-Stewart peeling with conditioned loop breakers instead of enumeration, so pedigrees with loops of more than 31 individuals (at most 128, at most 8 loop breakers) can be run. Posteriors equal those of -method 1 to 1e-9 relative; on a pedigree without loops the output is that of -method 2. Not with -familyBN."},
         {"-familyBN\t", "(this implementation) With -method 1: compute the Bayesian network of each family of the ped file on its own, for ped files of any size and families with loops (at most 31 members each). Members' posteriors equal those of the whole-file network except where its product of all members' probabilities leaves the double range."},
     };
     for (auto &r : rows) cout << r[0] << r[1] << endl << endl;
@@ -103,7 +104,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set family." << endl;
             return -1;
         }
-        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3, opt.peel_loops && opt.method == 1)) {
             cout << "Cannot set family." << endl;
             return -1;
         }
@@ -124,7 +125,7 @@ static int run(int argc, char *argv[]) {
             cout << "Cannot set Family." << endl;
             return -1;
         }
-        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3)) {
+        if (!check_family(ped, opt.family_bn && opt.method == 1, opt.method == 3, opt.peel_loops && opt.method == 1)) {
             cout << "Cannot set Family." << endl;
             return -1;
         }

@@ -141,6 +141,10 @@ int common_option(Scanner &sc, const std::string &opt, CommonOptions &o) {
         o.family_bn = true;
         return 1;
     }
+    if (opt == "peelLoops") {
+        o.peel_loops = true;
+        return 1;
+    }
     if (opt == "seed" && sc.value_follows()) {
         o.seed = std::strtoull(sc.take(), nullptr, 10);
         return 1;

@@ -22,6 +22,7 @@ struct CommonOptions {
     int device = 0;                 // -device k | a,b,c | all   CUDA device(s); a batch is split between several
     std::vector<int> devices;       //   (filled from -device; empty = {device})
     unsigned long long seed = 1;    // -seed n     Philox key of the Gibbs sampler
+    bool peel_loops = false;        // -peelLoops  with -method 1: exact BN posteriors by conditioned peeling (FS_METHOD_BN_PEEL)
     bool family_bn = false;         // -familyBN   with -method 1: each family of the ped file is its own Bayesian network
 };
 

@@ -145,6 +145,11 @@ struct fs_engine {
     int bn_rc = FS_OK;
     std::string bn_err;
 
+    BnPeelParams bn_peel; // FS_METHOD_BN_PEEL: the conditioned message program (host/bn_peel.hpp)
+    int bn_peel_rc = FS_OK;
+    std::string bn_peel_err;
+    int bn_peel_tb = 0;
+
     McmcParams mcmc;
     int mcmc_rc = FS_OK;
     std::string mcmc_err;
@@ -362,6 +367,9 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
                                   " families: only Elston-Stewart (-method 2) runs on ped files over " +
                                   std::to_string(FS_MAX_MEMBERS) + " members";
         e->mcmc_err += " (the Gibbs sampler on cohorts is fs_create_cohort_mcmc)";
+        e->bn_peel_rc = FS_E_ARG;
+        e->bn_peel_err = "conditioned peeling (method 4, -method 1 -peelLoops) runs on fs_create / fs_create_multi engines only, "
+                         "not on " + std::string(who) + " engines";
         if (mode == FamilyMode::BN) {
             e->cohort_bn = true;
             e->bn_rc = FS_OK;
@@ -430,6 +438,8 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
         }
         e->bn.C = C;
         e->bn_rc = build_bn_plan(e->ped, e->bn.plan, e->bn_err);
+        e->bn_peel.C = C;
+        e->bn_peel_rc = build_bn_peel_program(e->ped, e->bn_peel.peel, e->bn_peel_err);
         e->mcmc.C = C;
         e->mcmc_rc = build_mcmc_plan(e->ped, e->mcmc.plan, e->mcmc_err);
         if (const char *env = std::getenv("FAMSEQ_MCMC_JIT")) e->jit.mode = env[0] == '0' ? 0 : (env[0] == '1' ? 1 : 2);
@@ -460,6 +470,14 @@ static int create_engine(const fs_pedigree *ped, const fs_params *params, int de
             if (e->es_tb == 0) {
                 e->es_rc = FS_E_TOO_LARGE;
                 e->es_err = "pedigree too large for the ES kernel: message scratch exceeds shared memory";
+            }
+        }
+        if (e->bn_peel_rc == FS_OK && !families) {
+            e->bn_peel_tb = bn_peel_pick_block(e->bn_peel, e->smem_limit);
+            if (e->bn_peel_tb == 0) {
+                e->bn_peel_rc = FS_E_TOO_LARGE;
+                e->bn_peel_err = "pedigree too large for conditioned peeling (-method 1 -peelLoops): the vector file of " +
+                                 std::to_string(e->bn_peel.peel.n_vectors) + " genotype vectors per variant exceeds shared memory";
             }
         }
         if (e->bn_rc == FS_OK && !families && bn_smem_bytes(e->bn) > e->smem_limit) {
@@ -730,6 +748,29 @@ int fs_get_es_program(const fs_engine *e, uint32_t *words, int32_t capacity, int
     return FS_OK;
 }
 
+int fs_get_bn_peel_program(const fs_engine *e, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
+                           int32_t *breaker_rows, int32_t breaker_capacity, int32_t *n_breakers, int32_t *clamp_slots) {
+    if (!e) return fail(FS_E_ARG, "fs_get_bn_peel_program: null engine");
+    if (e->bn_peel_rc != FS_OK) return fail(e->bn_peel_rc, e->bn_peel_err);
+    const BnPeelProgram &p = e->bn_peel.peel;
+    if (n_words) *n_words = p.prog.n_words;
+    if (n_slots) *n_slots = p.prog.n_slots;
+    if (n_breakers) *n_breakers = p.n_breakers;
+    if (words) {
+        if (capacity < p.prog.n_words) return fail(FS_E_ARG, "fs_get_bn_peel_program: buffer too small");
+        std::memcpy(words, p.prog.words, sizeof(uint32_t) * (size_t)p.prog.n_words);
+    }
+    if ((breaker_rows || clamp_slots) && breaker_capacity < p.n_breakers) return fail(FS_E_ARG, "fs_get_bn_peel_program: breaker buffer too small");
+    for (int j = 0; j < p.n_breakers; j++) {
+        if (breaker_rows) breaker_rows[j] = p.breaker_row[j];
+        if (clamp_slots) {
+            clamp_slots[2 * j] = p.clamp_base + j;
+            clamp_slots[2 * j + 1] = p.clamp_base + p.n_breakers + j;
+        }
+    }
+    return FS_OK;
+}
+
 int fs_get_gibbs_kernel(const fs_engine *e, int compile, char *text, size_t capacity, size_t *text_len, size_t *cubin_bytes) {
     if (!e) return fail(FS_E_ARG, "fs_get_gibbs_kernel: null engine");
     if (e->mcmc_rc != FS_OK) return fail(e->mcmc_rc, e->mcmc_err);
@@ -915,10 +956,11 @@ static int ensure_pl_table(fs_engine *e, cudaStream_t stream) {
 static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t rep, uint64_t seed, int64_t v_offset,
                     cudaStream_t stream, double *lk_scratch = nullptr, double *single_scratch = nullptr) {
     if (B.V == 0) return FS_OK;
-    if (method != FS_METHOD_ES && method != FS_METHOD_BN && method != FS_METHOD_MCMC)
-        return fail(FS_E_ARG, "method must be 1 (BN), 2 (ES) or 3 (MCMC)");
+    if (method != FS_METHOD_ES && method != FS_METHOD_BN && method != FS_METHOD_MCMC && method != FS_METHOD_BN_PEEL)
+        return fail(FS_E_ARG, "method must be 1 (BN), 2 (ES), 3 (MCMC) or 4 (BN by conditioned peeling)");
     if (method == FS_METHOD_ES && e->es_rc != FS_OK) return fail(e->es_rc, e->es_err);
     if (method == FS_METHOD_BN && e->bn_rc != FS_OK) return fail(e->bn_rc, e->bn_err);
+    if (method == FS_METHOD_BN_PEEL && e->bn_peel_rc != FS_OK) return fail(e->bn_peel_rc, e->bn_peel_err);
     if (method == FS_METHOD_MCMC) {
         if (e->mcmc_rc != FS_OK) return fail(e->mcmc_rc, e->mcmc_err);
         if (burn < 0 || rep <= 0) return fail(FS_E_ARG, "MCMC needs burn >= 0 and rep >= 1");
@@ -1003,6 +1045,9 @@ static int dispatch(fs_engine *e, int method, BatchPtrs B, int32_t burn, int32_t
     }
     case FS_METHOD_BN:
         krc = launch_bn(e->bn, B, e->sm_count, stream);
+        break;
+    case FS_METHOD_BN_PEEL:
+        krc = launch_bn_peel(e->bn_peel, B, e->bn_peel_tb, stream);
         break;
     case FS_METHOD_MCMC: {
         GibbsJitState &J = e->jit;

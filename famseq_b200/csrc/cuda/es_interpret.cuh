@@ -35,14 +35,37 @@ template <int TB> struct EsThread {
 // zero (the reference returns false there, family.cpp:1305-1310).  `prog.word(pc)` is word pc of the program and
 // `prog.col(c)` the output column of its input column c: the kernel parameters and the identity for es_kernel, a family's
 // program and column map in global memory for the cohort kernel (es_cohort_kernel.cu).
-template <bool X, int TB, class Program>
-__device__ bool es_interpret(const RunConstants &C, const Program &prog, const EsThread<TB> &t, double *post_row, uint8_t *gt_row) {
+// ACC: the conditioned program of bn_peel_kernel.cu, whose ES_OP_ACC stores (acc_first) or adds each member's
+// unnormalised marginal into its accumulator; it exists only in that instantiation.
+template <bool X, int TB, class Program, bool ACC = false>
+__device__ bool es_interpret(const RunConstants &C, const Program &prog, const EsThread<TB> &t, double *post_row, uint8_t *gt_row,
+                             bool acc_first = true) {
     bool failed = false;
     int pc = 0;
     for (;;) {
         const uint32_t w0 = prog.word(pc);
         const uint32_t op = w0 & 0xffu;
         if (op == ES_OP_END) break;
+        if constexpr (ACC) {
+            if (op == ES_OP_ACC) {
+                const uint32_t w1 = prog.word(pc + 1), w2 = prog.word(pc + 2), acc = (w0 >> 8) & 0xffffu;
+                double m[3], l[3], a[3];
+                t.load(w1 & 0xffffu, m);
+                t.load(w1 >> 16, l);
+                t.load(w2 & 0xffffu, a);
+#pragma unroll
+                for (int g = 0; g < 3; g++) m[g] = (m[g] * l[g]) * a[g];
+                if (!acc_first) { // never 0.0 + v on the first peel: it would turn a -0.0 into +0.0
+                    double s[3];
+                    t.load(acc, s);
+#pragma unroll
+                    for (int g = 0; g < 3; g++) m[g] = s[g] + m[g];
+                }
+                t.store(acc, m);
+                pc += 3;
+                continue;
+            }
+        }
         if (op == ES_OP_MUL) {
             const uint32_t w1 = prog.word(pc + 1);
             double a[3], b[3];

@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <vector>
 
+#include "../host/bn_peel.hpp"
 #include "../host/bn_plan.hpp"
 #include "../host/es_program.hpp"
 #include "../host/mcmc_plan.hpp"
@@ -23,6 +24,15 @@ struct EsParams {
 size_t es_smem_bytes(const EsParams &P, int tb);
 int es_pick_block(const EsParams &P, size_t smem_limit);
 cudaError_t launch_es(const EsParams &P, const BatchPtrs &B, int tb, cudaStream_t stream);
+
+// ---- Bayesian network by conditioned peeling (bn_peel_kernel.cu) ---------------------------------------------
+struct BnPeelParams {
+    RunConstants C;
+    BnPeelProgram peel;
+};
+// es_pick_block's rule for the conditioned program's vector file; 0 when not even 32 variants fit.
+int bn_peel_pick_block(const BnPeelParams &P, size_t smem_limit);
+cudaError_t launch_bn_peel(const BnPeelParams &P, const BatchPtrs &B, int tb, cudaStream_t stream);
 
 // ---- Elston-Stewart, nuclear families (es_nuclear_kernel.cu) -------------------------------------------
 constexpr int ES_NUCLEAR_MAX_CHILDREN = 5;

@@ -41,10 +41,11 @@ struct Op {
 
 class Compiler {
   public:
-    explicit Compiler(const Pedigree &p) : ped(p), ant_slot(p.n, -1), ant_busy(p.n, 0) {}
+    Compiler(const Pedigree &p, const EsConditioning *c) : ped(p), cond(c), ant_slot(p.n, -1), ant_busy(p.n, 0) {}
 
     bool run(std::string &err) {
-        for (int i = 0; i < ped.n && !loop; i++) {
+        const int n_fin = cond ? cond->n_real : ped.n; // founder copies have no marginal of their own
+        for (int i = 0; i < n_fin && !loop; i++) {
             // family.cpp:1296-1301: postTmp = (prod_k pos(i,.,spouse k)) * lk(i,.) * ant(i,.)
             std::vector<Ref> below;
             for (int sp : ped.spouses[i]) below.push_back(pos(i, sp));
@@ -54,6 +55,10 @@ class Compiler {
             f.b = lk(i);
             f.c = ant(i);
             f.col = ped.col_of[i];
+            if (cond) {
+                f.op = ES_OP_ACC;
+                f.dst = cond->acc_fixed[i]; // a reserved vector, not a virtual slot
+            }
             ops.push_back(f);
         }
         if (loop) {
@@ -69,6 +74,7 @@ class Compiler {
 
   private:
     const Pedigree &ped;
+    const EsConditioning *cond;
     std::vector<int> ant_slot;
     std::vector<char> ant_busy;
     std::map<std::pair<int, int>, int> pos_slot;
@@ -78,7 +84,10 @@ class Compiler {
 
     Ref lk(int i) const {
         Ref r;
-        if (ped.col_of[i] >= 0) {
+        if (cond && cond->lk_fixed[i] >= 0) {
+            r.kind = ES_REF_FIXED;
+            r.index = cond->lk_fixed[i];
+        } else if (ped.col_of[i] >= 0) {
             r.kind = ES_REF_LK;
             r.index = ped.col_of[i];
         }
@@ -121,6 +130,11 @@ class Compiler {
     Ref ant(int i) {
         if (ped.founder(i)) {
             Ref r;
+            if (cond && cond->ant_fixed[i] >= 0) {
+                r.kind = ES_REF_FIXED;
+                r.index = cond->ant_fixed[i];
+                return r;
+            }
             r.kind = ES_REF_PRIOR;
             r.index = ped.male[i];
             return r;
@@ -201,10 +215,10 @@ template <class F> void for_each_ref(Op &o, F f) {
 
 } // namespace
 
-int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err) {
+int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err, const EsConditioning *cond) {
     out = EsProgram();
     out.n_cols = ped.s();
-    Compiler c(ped);
+    Compiler c(ped, cond);
     if (!c.run(err)) return FS_E_LOOP;
 
     // Liveness-based slot reuse: a virtual slot dies after its last reader; the destination of an
@@ -222,7 +236,7 @@ int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err) {
     int n_phys = 0;
     for (int k = 0; k < nops; k++) {
         Op &o = c.ops[k];
-        if (o.dst >= 0) {
+        if (o.dst >= 0 && o.op != ES_OP_ACC) {
             if (free_list.empty()) {
                 phys[o.dst] = n_phys++;
             } else {
@@ -237,7 +251,7 @@ int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err) {
         for_each_ref(o, [&](Ref &r) {
             if (r.kind == ES_REF_SLOT) r.index = phys[r.index];
         });
-        if (o.dst >= 0) o.dst = phys[o.dst];
+        if (o.dst >= 0 && o.op != ES_OP_ACC) o.dst = phys[o.dst];
     }
     out.n_slots = n_phys;
     out.n_ops = nops;
@@ -248,17 +262,20 @@ int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err) {
 
     // Operand encoding: index of a 3-vector in the per-variant vector file the kernel keeps in shared memory --
     // [0, S) likelihood rows of the input columns, [S, S + n_slots) message scratch, then the founder prior of a
-    // non-male member, the founder prior of a male member, and the vector of ones.
+    // non-male member, the founder prior of a male member, and the vector of ones; a conditioned program's reserved
+    // vectors follow.
     const uint32_t S = (uint32_t)ped.s(), first_slot = S, special = S + (uint32_t)n_phys;
+    const uint32_t n_fixed = cond ? (uint32_t)cond->n_fixed : 0u;
     auto enc = [&](const Ref &r) -> uint32_t {
         switch (r.kind) {
         case ES_REF_LK: return (uint32_t)r.index;
         case ES_REF_SLOT: return first_slot + (uint32_t)r.index;
         case ES_REF_PRIOR: return special + (r.index ? 1u : 0u);
+        case ES_REF_FIXED: return special + 3u + (uint32_t)r.index;
         default: return special + 2u;
         }
     };
-    if (special + 3u >= 0xffffu) {
+    if (special + 3u + n_fixed >= 0xffffu) {
         err = "pedigree too large for the ES message program (vector file)";
         return FS_E_TOO_LARGE;
     }
@@ -284,6 +301,11 @@ int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err) {
             break;
         case ES_OP_FIN:
             w.push_back(ES_OP_FIN | (o.col >= 0 ? 1u << 8 : 0u) | (uint32_t)(o.col >= 0 ? o.col : 0) << 9);
+            w.push_back(enc(o.a) | enc(o.b) << 16);
+            w.push_back(enc(o.c));
+            break;
+        case ES_OP_ACC:
+            w.push_back(ES_OP_ACC | (special + 3u + (uint32_t)o.dst) << 8);
             w.push_back(enc(o.a) | enc(o.b) << 16);
             w.push_back(enc(o.c));
             break;

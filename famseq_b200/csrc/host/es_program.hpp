@@ -8,6 +8,7 @@
 
 #include <cstdint>
 #include <string>
+#include <vector>
 
 #ifdef __CUDACC__
 #define FS_HD __host__ __device__
@@ -31,6 +32,7 @@ enum EsRefKind : uint32_t {
     ES_REF_SLOT = 1,  // per-thread scratch 3-vector `index`
     ES_REF_LK = 2,    // likelihood of input column `index`
     ES_REF_PRIOR = 3, // founder prior; index 1 = male (uses the chrX male prior on X), 0 = otherwise
+    ES_REF_FIXED = 4, // conditioned program (host/bn_peel.hpp): reserved vector `index` behind the three special vectors
 };
 FS_HD constexpr uint32_t es_ref(EsRefKind k, uint32_t index) { return ((uint32_t)k << 13) | (index & 0x1fffu); }
 FS_HD constexpr uint32_t es_ref_kind(uint32_t r) { return (r >> 13) & 7u; }
@@ -53,6 +55,10 @@ enum EsOpcode : uint32_t {
     // otherwise, when the member is sequenced, post[col] = v / sum and gt[col] = arg max.
     // word0 = opcode | has_col<<8 | col<<9 ; word1 = M | lk<<16 ; word2 = ant
     ES_OP_FIN = 4,
+    // conditioned peeling (host/bn_peel.hpp) in place of FIN: v = (M (*) lk) (*) ant is stored into (first peel) or added
+    // to (later peels) the accumulator vector `acc`; no normalisation and no row-sum test.
+    // word0 = opcode | acc<<8 ; word1 = M | lk<<16 ; word2 = ant
+    ES_OP_ACC = 5,
     ES_OP_END = 0,
 };
 
@@ -66,8 +72,18 @@ struct EsProgram {
     uint32_t words[ES_MAX_WORDS];
 };
 
+// Overrides of the conditioned program (host/bn_peel.cpp), in reserved vectors (ES_REF_FIXED, numbered from 0 right behind
+// the three special vectors).  Members [0, n_real) are the pedigree's own; rows from n_real on are founder copies.
+struct EsConditioning {
+    int n_real = 0;
+    std::vector<int> lk_fixed;  // [n] reserved vector replacing lk(i) (a breaker's clamped likelihood), or -1
+    std::vector<int> ant_fixed; // [n] reserved vector replacing a founder copy's prior (the clamp indicator), or -1
+    std::vector<int> acc_fixed; // [n_real] accumulator of member i: its FIN becomes ES_OP_ACC into this vector
+    int n_fixed = 0;            // reserved vectors in all
+};
+
 // Host entry point of the pedigree compiler (es_program.cpp).  Returns FS_OK, FS_E_LOOP (pedigree is not
-// peelable) or FS_E_TOO_LARGE; `err` receives the text.
-int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err);
+// peelable) or FS_E_TOO_LARGE; `err` receives the text.  With `cond`, the conditioned program of bn_peel.cpp.
+int compile_es_program(const Pedigree &ped, EsProgram &out, std::string &err, const EsConditioning *cond = nullptr);
 
 } // namespace famseq

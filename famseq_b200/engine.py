@@ -19,7 +19,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libfamseq_b200.so")
 
-BN, ES, MCMC = 1, 2, 3
+BN, ES, MCMC, BN_PEEL = 1, 2, 3, 4  # BN_PEEL: BN's answer by conditioned peeling (-method 1 -peelLoops)
 FLAG_KNOWN, FLAG_CHRX = 1, 2
 
 FS_ERRORS = {
@@ -130,6 +130,8 @@ def lib() -> ctypes.CDLL:
         L.fs_last_kernel_ms.argtypes = [P]
         L.fs_get_es_program.restype = ctypes.c_int
         L.fs_get_es_program.argtypes = [P, P, I32, P, P]
+        L.fs_get_bn_peel_program.restype = ctypes.c_int
+        L.fs_get_bn_peel_program.argtypes = [P, P, I32, P, P, P, I32, P, P]
         L.fs_bench_fp64_tflops.restype = ctypes.c_int
         L.fs_bench_fp64_tflops.argtypes = [ctypes.c_int, P]
         _lib = L
@@ -142,7 +144,7 @@ EXPORTED_SYMBOLS = ["fs_default_params", "fs_device_count", "fs_create", "fs_des
                     "fs_create_multi", "fs_run_pl", "fs_run_pl_device", "fs_get_pl_table",
                     "fs_run_pl_phred", "fs_phred_encode", "fs_phred_text", "fs_phred_text_exact",
                     "fs_create_families", "fs_get_families", "fs_create_cohort", "fs_get_family_program", "fs_create_cohort_bn",
-                    "fs_create_cohort_mcmc"]
+                    "fs_create_cohort_mcmc", "fs_get_bn_peel_program"]
 
 
 def _check(rc: int) -> None:
@@ -286,6 +288,17 @@ class Engine:
         words = np.zeros(n_words.value, np.uint32)
         _check(lib().fs_get_es_program(self._h, _ptr(words), n_words.value, None, None))
         return words, int(n_slots.value)
+
+    def bn_peel_program(self):
+        """(words, n_slots, breaker_rows, clamp_slots) of the conditioned program of BN_PEEL (fs_get_bn_peel_program):
+        clamp_slots[j] = (vector of breaker j's clamped likelihood, vector of its indicator)."""
+        n_words, n_slots, k = ctypes.c_int32(0), ctypes.c_int32(0), ctypes.c_int32(0)
+        _check(lib().fs_get_bn_peel_program(self._h, None, 0, ctypes.byref(n_words), ctypes.byref(n_slots), None, 0,
+                                            ctypes.byref(k), None))
+        words, rows, clamps = np.zeros(n_words.value, np.uint32), np.zeros(k.value, np.int32), np.zeros((k.value, 2), np.int32)
+        _check(lib().fs_get_bn_peel_program(self._h, _ptr(words), n_words.value, None, None, _ptr(rows), k.value, None,
+                                            _ptr(clamps)))
+        return words, int(n_slots.value), rows, clamps
 
     def es_kernel(self, compile: bool = False):
         """(text, cubin_bytes): the CUDA C++ generated for this pedigree's Elston-Stewart peeling, or the compile log."""

@@ -41,7 +41,18 @@ extern "C" {
 
 #define FS_ABI_VERSION 2
 
-enum fs_method { FS_METHOD_BN = 1, FS_METHOD_ES = 2, FS_METHOD_MCMC = 3 }; /* the CLI's -method 1|2|3 */
+/* the CLI's -method 1|2|3; FS_METHOD_BN_PEEL is -method 1 -peelLoops.
+ * FS_METHOD_BN_PEEL: the Bayesian network's answer -- each member's normalised exact marginal -- computed by Elston-Stewart
+ * peeling with conditioned loop breakers (loop-cutset conditioning) instead of enumerating 3^n configurations, so it takes
+ * looped pedigrees of any size fs_create takes (<= 128 members).  K breakers (K <= the pedigree's cycle rank, 0 for a
+ * loop-free pedigree) each hand their marriages on loops to founder copies; the loop-free result is peeled once for each of
+ * the 3^K genotype assignments of the breakers and the unnormalised marginals are added up.  Posteriors are those of
+ * FS_METHOD_BN to 1e-9 relative; on a loop-free pedigree every output byte is that of FS_METHOD_ES.  Status 1 as BN: an
+ * individual-only row sum <= 0, an unsequenced member's failing prior, or a member whose accumulated marginal sums to <= 0
+ * (where the unscaled total likelihood underflows).  fs_create accepts the same pedigrees as without it; a run returns
+ * FS_E_TOO_LARGE, with the reason, for a pedigree that needs more than 8 breakers, a program over ES_MAX_WORDS words or, on
+ * a device, a vector file over shared memory.  Cohort engines refuse it with FS_E_ARG. */
+enum fs_method { FS_METHOD_BN = 1, FS_METHOD_ES = 2, FS_METHOD_MCMC = 3, FS_METHOD_BN_PEEL = 4 };
 
 enum fs_flag { FS_FLAG_KNOWN = 1, /* VCF ID != "."  (file.cpp:476-480) */
                FS_FLAG_CHRX = 2 /* CHROM in {X,chrX,CHRX} (file.cpp:482-486) */ };
@@ -270,6 +281,15 @@ int fs_get_tables(const fs_engine *e, double *pcp2, double *pcp2_xf, double *pcp
  * `words` (capacity in words); *n_words / *n_slots receive its length and scratch size.  Introspection only:
  * tests interpret it on the CPU to check the pedigree compiler without a GPU.  FS_E_LOOP on looped pedigrees. */
 int fs_get_es_program(const fs_engine *e, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots);
+
+/* The conditioned program of FS_METHOD_BN_PEEL (host/bn_peel.hpp): its words (the format of fs_get_es_program plus
+ * ES_OP_ACC), *n_words, *n_slots, the ped rows of its *n_breakers loop breakers in breaker_rows (breaker_capacity entries)
+ * and, in clamp_slots[2 * breaker_capacity], the vector-file index of each breaker's clamped likelihood and of its
+ * indicator.  The accumulators follow the indicators: input column c's member, then the unsequenced members in ped order.
+ * Every pointer may be NULL.  Introspection: tests interpret the program on the CPU.  The run's error where the program is
+ * refused. */
+int fs_get_bn_peel_program(const fs_engine *e, uint32_t *words, int32_t capacity, int32_t *n_words, int32_t *n_slots,
+                           int32_t *breaker_rows, int32_t breaker_capacity, int32_t *n_breakers, int32_t *clamp_slots);
 
 /* The Gibbs sampler of large MCMC batches is a kernel the engine writes for this one pedigree and compiles for
  * sm_100a at run time (NVRTC; csrc/cuda/gibbs_jit.cu) -- it replaces the same reference functions as the table-driven
